@@ -1,6 +1,6 @@
 """bench.py — YOLOX-s 640^2 images/s (fwd + decode + NMS) on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +23,8 @@ per GPU (weak scaling: the batch is sharded by image, no data-path collective).
   --train   : config 4, one training step (fwd-train + SimOTA + losses + backward + gradient all-reduce + SGD)
   --global-batch G : strong scaling, G images per step split over the ranks (config 3: --model yolox_l --dtype fp16
               --global-batch 512)
+  --dump-outputs DIR : after the timed steps, what the last one returned to its caller as DIR/<name>.npy (see
+              dump_outputs), so that two builds can be compared output for output on the same seeded inputs
 """
 from __future__ import annotations
 
@@ -37,6 +39,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 GFLOP_PER_IMAGE = {"yolox_s": 26.686, "yolox_m": 73.530, "yolox_l": 155.293, "yolox_x": 281.410,
                    "yolox_tiny": 6.413, "yolox_nano": 1.045}   # BASELINE.md section 2 (conv 2*MAC)
@@ -66,7 +69,14 @@ def parse():
                     help="--train: memory format of the module and its input in our arm (cuDNN's 16-bit kernels are NHWC; "
                          "our BatchNorm + activation kernels take both)")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra legs (conf 0.01, config 5, torch GPU reference)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed inference step to DIR/<name>.npy (rank 0's images)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.train or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the inference step of --impl ours")
+    return args
 
 
 def peaks():
@@ -360,6 +370,39 @@ def parity_check(model, engine, args) -> dict:
             "parity_how": "last timed step's detections == YoloxModule.forward + postprocess on the same batch (torch.equal per image)"}
 
 
+DUMP_BYTES = 64 << 20                   # --dump-outputs: at most this much in all
+PRED_SAMPLE_ROWS = 65536                # head-output rows kept in the dump (seeded sample; 22 MB at 85 columns)
+
+
+def dump_outputs(out_dir: str, engine, max_det: int) -> dict:
+    """--dump-outputs: what the timed step hands its caller (YoloxModule.detect returns dets / det_idx / det_count, the
+    engine's forward the head output), copied after the timed region and written as float32 / float64 .npy files:
+      dets [B, K, 7] f32, det_idx [B, K] f64, det_count [B] f64: K is the largest kept count of the batch (at most max_det);
+          the rows past an image's own count are zero in dets and -1 in det_idx (the buffers leave them undefined)
+      pred_rows [N, 5 + nc] f32: the rows pred_rows_index [N] f64 (row numbers of the flattened [B * A] head output) of a
+          fixed, seeded sample of the head output, which is too large to store whole (183 MB for yolox_s at batch 64)."""
+    import numpy as np
+    import torch
+
+    count = engine.det_count.cpu()
+    kept = count.clamp(max=max_det).long()
+    k = int(kept.max().item()) if kept.numel() else 0
+    live = torch.arange(k)[None, :] < kept[:, None]
+    dets = torch.where(live[..., None], engine.dets[:, :k].cpu(), torch.zeros(()))
+    idx = torch.where(live, engine.det_idx[:, :k].cpu(), torch.full((), -1, dtype=torch.int64))
+    pred = engine.pred.reshape(-1, engine.pred.shape[-1])
+    left = DUMP_BYTES - 4 * dets.numel() - 8 * idx.numel() - 8 * count.numel()
+    n = max(0, min(pred.shape[0], PRED_SAMPLE_ROWS, left // (4 * pred.shape[1] + 8)))
+    rows = np.sort(np.random.default_rng(0).choice(pred.shape[0], size=n, replace=False))
+    out = {"dets": dets.float().numpy(), "det_idx": idx.double().numpy(), "det_count": count.double().numpy(),
+           "pred_rows": pred[torch.from_numpy(rows).to(pred.device)].float().cpu().numpy(),
+           "pred_rows_index": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: list(a.shape) for name, a in out.items()}
+
+
 def extra_conf_leg(args, model, dev_in, conf: float, steps: int) -> dict:
     """The same step at another score threshold (0.01 = the evaluator's test_conf, yolox/config.py:115)."""
     import torch
@@ -614,6 +657,9 @@ def run_ours(args):
     barrier()
     value = total_images * args.steps / (ms / 1e3)
     last = eng[(args.steps - 1) % 2]
+    if args.dump_outputs and rank == 0:
+        shapes = dump_outputs(args.dump_outputs, last, args.max_det)
+        print(f"# outputs of the last timed step written to {args.dump_outputs}: {shapes}", file=sys.stderr)
     kept = int(last.det_count.clamp(max=args.max_det).sum().item())
     kept_true_mean = float(last.det_count.float().mean().item())
     scores = last.pred[..., 4] * last.pred[..., 5:].max(-1).values

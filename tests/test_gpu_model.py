@@ -207,7 +207,7 @@ def test_engine_cache_survives_deepcopy_and_weight_changes(cuda):
         copy.deepcopy(next(iter(model._engines.values())))
 
 
-def test_config1_nano_416_user_api_on_gpu():
+def test_config1_nano_416_user_api_on_gpu(cuda):
     """BASELINE.json config 1 on the GPU path: yolox_nano (depthwise) 416x416 batch 1, fp32 verification mode within 1e-3 of
     the reference's CPU output (or the conditioning ceiling of the same graph in torch-CUDA fp32), bf16 at the torch-bf16
     ceiling; YoloxProcessor.postprocess on the reference's own head tensor returns the reference's Detections exactly."""
@@ -217,7 +217,7 @@ def test_config1_nano_416_user_api_on_gpu():
 
     g = np.load(Path(__file__).resolve().parent / "golden" / "config1.npz")
     c = cases.CONFIG1
-    dev = torch.device("cuda", 0)
+    dev = cuda
     img = Image.fromarray(cases.config1_image())
     proc = yx.YoloxProcessor(c["name"])
     proc.nms_variant = "auto_cpu"                  # the fixture was produced by the reference on CPU (torchvision's CPU rule)

@@ -123,3 +123,38 @@ def test_set_match_comparator():
     assert match_sets([a], [b]) == 1
     assert match_sets([a, None], [b, a]) == 1 and match_sets([a], [None]) == 0
     assert match_sets([a], [np.concatenate([a, a])]) == 3          # one-to-one: duplicates do not count twice
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs on an engine's output buffers: float32 / float64 arrays within 64 MB, the detections of each
+    image up to its kept count (at most max_det) and cleared after it, the same seeded sample of head-output rows every run."""
+    import types
+
+    import bench
+
+    B, A, nc, max_det = 8, 8400, 80, 1000
+    g = torch.Generator().manual_seed(0)
+    eng = types.SimpleNamespace(det_count=torch.randint(0, 50, (B,), dtype=torch.int32, generator=g),
+                                dets=torch.randn(B, max_det, 7, generator=g),
+                                det_idx=torch.randint(0, B * A, (B, max_det), generator=g),
+                                pred=torch.randn(B, A, 5 + nc, generator=g))
+    eng.det_count[1] = max_det + 5
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), eng, max_det)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["det_count.npy", "det_idx.npy", "dets.npy", "pred_rows.npy", "pred_rows_index.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 64 << 20
+    out = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert out[f[:-4]].dtype in (np.float32, np.float64)
+        assert np.array_equal(out[f[:-4]], np.load(tmp_path / "b" / f))
+    np.testing.assert_array_equal(out["det_count"], eng.det_count.numpy())
+    kept = np.minimum(eng.det_count.numpy(), max_det)
+    assert out["dets"].shape == (B, max_det, 7) and out["det_idx"].shape == (B, max_det)
+    for b, k in enumerate(kept):
+        np.testing.assert_array_equal(out["dets"][b, :k], eng.dets[b, :k].numpy())
+        np.testing.assert_array_equal(out["det_idx"][b, :k], eng.det_idx[b, :k].numpy())
+        assert (out["dets"][b, k:] == 0).all() and (out["det_idx"][b, k:] == -1).all()
+    rows = out["pred_rows_index"].astype(np.int64)
+    assert len(rows) == bench.PRED_SAMPLE_ROWS < B * A and len(np.unique(rows)) == len(rows)
+    np.testing.assert_array_equal(out["pred_rows"], eng.pred.reshape(B * A, 5 + nc)[rows].numpy())
