@@ -123,6 +123,13 @@ typedef struct yx_conv_desc {
 
 /* tcgen05/TMEM/TMA implicit GEMM for bf16/fp16; routes YX_FP32 to the SIMT kernel. */
 int yx_conv_bn_act_fwd(const yx_conv_desc* d, void* stream);
+/* Runs the launch selection of yx_conv_bn_act_fwd for `d` without launching (needs a device: it encodes the tensor
+ * maps). Fills up to `capacity` ints and returns the count, or a negative yx_status:
+ *   mode (0 per-tap ring, 1 halo, 2 stride-2 planes), flat, b_resident, G, ctas_per_sm, epi_groups, acc_stages, a_slots,
+ *   stages, BN, n_tiles, m_tiles, num_tiles, grid, tw, th.
+ * CTA i of the halo / planes modes owns the units [num_tiles*i/grid, num_tiles*(i+1)/grid); the per-tap ring hands
+ * tile t to CTA t % grid. */
+int yx_conv_schedule(const yx_conv_desc* d, int32_t* info, int32_t capacity);
 /* ------------------------------------------------------------------------------------------
  * Fused Bottleneck: y = [x +] act(bn2(conv3x3(act(bn1(conv1x1(x))))))  in one kernel
  *   replaces Bottleneck.forward (yolox/models/network_blocks.py:77-99: conv1 1x1, conv2 3x3,

@@ -71,6 +71,7 @@ SIGNATURES = {
     "yx_device_check": (C.c_int, [C.c_int]),
     "yx_conv_bn_act_fwd": (C.c_int, [C.POINTER(ConvDesc), _P]),
     "yx_conv_bn_act_fwd_simt": (C.c_int, [C.POINTER(ConvDesc), _P]),
+    "yx_conv_schedule": (C.c_int, [C.POINTER(ConvDesc), _P, _I32]),
     "yx_bottleneck_fwd": (C.c_int, [C.POINTER(BneckDesc), _P]),
     "yx_bottleneck_supported": (C.c_int, [C.POINTER(BneckDesc)]),
     "yx_dwconv3x3_bn_act_fwd": (C.c_int, [_P, _I64, _P, _P, _P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P]),

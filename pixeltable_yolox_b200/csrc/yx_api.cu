@@ -16,6 +16,7 @@ struct ConvTcParams;
 struct ConvTcLaunch;
 int conv_tc_prepare(const yx_conv_desc* d, ConvTcLaunch* L);
 int conv_tc_launch(const ConvTcLaunch* L, cudaStream_t stream);
+int conv_tc_schedule(const yx_conv_desc* d, int32_t* info, int capacity);
 int conv_simt_launch(const yx_conv_desc* d, cudaStream_t stream);
 int focus_launch(const void* img, int img_dtype, void* out, long long out_ld, int out_dtype, int batch, int h, int w, cudaStream_t s);
 int spp_launch(void* buf, long long ld, int batch, int h, int w, int c, int dtype, cudaStream_t s);
@@ -263,6 +264,14 @@ int yx_conv_bn_act_fwd(const yx_conv_desc* d, void* stream) {
   if (rc == YX_OK) rc = conv_tc_launch(L, (cudaStream_t)stream);
   conv_tc_free(L);
   return rc;
+}
+
+int yx_conv_schedule(const yx_conv_desc* d, int32_t* info, int32_t capacity) {
+  int rc = require_device();
+  if (rc) return rc;
+  YX_REQUIRE(d != nullptr && (info != nullptr || capacity <= 0), YX_ERR_INVALID_ARG, "conv_schedule: null argument");
+  YX_REQUIRE(d->dtype != YX_FP32, YX_ERR_UNSUPPORTED, "conv_schedule: fp32 convs run on the SIMT kernel (no tile schedule)");
+  return conv_tc_schedule(d, info, capacity);
 }
 
 int yx_bottleneck_supported(const yx_bneck_desc* d) { return bneck_supported(d) ? 1 : 0; }

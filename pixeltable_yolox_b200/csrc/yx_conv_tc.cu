@@ -834,6 +834,7 @@ struct ConvTcLaunch {
   CUtensorMap map_a, map_b;
   ConvTcParams p;
   int grid;
+  int ctas;              // co-resident CTAs per SM the launch was sized for
   size_t smem;
 };
 
@@ -1208,6 +1209,7 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   p.mul_ohw = fast_div_mul(d->out_h * d->out_w);
   p.mul_ow = fast_div_mul(d->out_w);
   const int sms = num_sms() * ctas;
+  L->ctas = ctas;
   L->grid = p.num_tiles < sms ? p.num_tiles : sms;
   if (p.halo) {
     const int groups = p.num_tiles / p.G;     // never split a weight-sharing group when there is less than one per SM
@@ -1225,6 +1227,23 @@ ConvTcLaunch* conv_tc_alloc() {
   return reinterpret_cast<ConvTcLaunch*>(p);
 }
 void conv_tc_free(ConvTcLaunch* p) { free(p); }
+
+// The launch selection of conv_tc_prepare, without a launch (yx_conv_schedule): tests use it to show which mode, ring
+// depths and per-CTA tile ranges a shape exercises.
+int conv_tc_schedule(const yx_conv_desc* d, int32_t* info, int capacity) {
+  ConvTcLaunch* L = conv_tc_alloc();
+  YX_REQUIRE(L != nullptr, YX_ERR_INVALID_ARG, "conv_schedule: out of host memory");
+  const int rc = conv_tc_prepare(d, L);
+  int n = 0;
+  if (rc == YX_OK) {
+    const ConvTcParams& p = L->p;
+    const int32_t v[] = {p.halo, p.flat, p.b_resident, p.G, L->ctas, p.epi_groups, p.acc_stages, p.a_slots,
+                         p.stages, p.BN, p.n_tiles, p.m_tiles, p.num_tiles, L->grid, p.tw, p.th};
+    for (; n < (int)(sizeof(v) / sizeof(v[0])) && n < capacity; ++n) info[n] = v[n];
+  }
+  conv_tc_free(L);
+  return rc == YX_OK ? n : rc;
+}
 
 int conv_tc_launch(const ConvTcLaunch* L, cudaStream_t stream) {
   static bool attr_set_dev[kMaxDevices] = {};

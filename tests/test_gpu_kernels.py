@@ -92,9 +92,10 @@ def test_conv_two_destinations(cuda, k):
     assert (o2[..., :16] == 7).all()
 
 
-def _bneck_case(dev, B, H, W, c, dtype, use_add, act, in_off=0, out_off=0, seed=0):
-    """Fused Bottleneck against torch: fp32 math with the hidden tensor rounded to the 16-bit dtype, exactly
-    what the reference's two 16-bit BaseConvs do (network_blocks.py:77-99)."""
+def _bneck_run(dev, B, H, W, c, dtype, use_add, act, in_off=0, out_off=0, seed=0):
+    """Fused Bottleneck and its torch reference: fp32 math with the hidden tensor rounded to the 16-bit dtype, exactly
+    what the reference's two 16-bit BaseConvs do (network_blocks.py:77-99). Returns (kernel output as fp32, reference,
+    the whole output buffer, the kernel's inputs)."""
     g = torch.Generator().manual_seed(seed)
     x = torch.randn(B, H, W, c + 2 * in_off, generator=g).to(dev).to(dtype)
     w1 = (torch.randn(c, 1, c, generator=g) / c ** 0.5).to(dev).to(dtype)
@@ -110,8 +111,11 @@ def _bneck_case(dev, B, H, W, c, dtype, use_add, act, in_off=0, out_off=0, seed=
     y = f(F.conv2d(h, w2.float().reshape(c, 3, 3, c).permute(0, 3, 1, 2), b2, 1, 1))
     if use_add:
         y = y + xf
-    y = y.permute(0, 2, 3, 1)
-    got = ov.torch().float()
+    return ov.torch().float(), y.permute(0, 2, 3, 1), o, (xin, w1, b1, w2, b2)
+
+
+def _bneck_case(dev, B, H, W, c, dtype, use_add, act, in_off=0, out_off=0, seed=0):
+    got, y, o, _ = _bneck_run(dev, B, H, W, c, dtype, use_add, act, in_off, out_off, seed)
     if out_off:
         assert (o[..., :out_off] == 7).all() and (o[..., out_off + c:] == 7).all(), "wrote outside the channel slice"
     return ((got - y).abs() / y.abs().clamp_min(1.0)).max().item()
