@@ -247,7 +247,6 @@ int allreduce_sgd_ema_launch(const long long* table, const int* chunks, int n_ch
     p.peer_grad[q] = peer_grad[q]; p.peer_flag[q] = peer_flag[q];
   }
   p.flat_elems = flat_elems; p.rank = rank; p.world = world; p.state = state;
-  static const int coop = (getenv("YX_AR_COOP") && getenv("YX_AR_COOP")[0] == '0') ? 0 : 1;
   static int cap_dev[kMaxDevices] = {};
   int& cap = cap_dev[current_device_slot()];
   if (cap == 0) {
@@ -264,7 +263,7 @@ int allreduce_sgd_ema_launch(const long long* table, const int* chunks, int n_ch
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeCooperative;
   attr[0].val.cooperative = 1;
-  cfg.attrs = attr; cfg.numAttrs = coop;
+  cfg.attrs = attr; cfg.numAttrs = 1;
   YX_CUDA(cudaLaunchKernelEx(&cfg, allreduce_sgd_ema_kernel, p));
   return YX_OK;
 }

@@ -127,24 +127,6 @@ int num_sms() {
   return cached;
 }
 
-bool train_pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("YX_TRAIN_PDL");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v != 0;
-}
-
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("YX_PDL");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-
 static int require_device() {
   static int ok_dev[kMaxDevices] = {};         // checked once per device, not once per process
   int& ok = ok_dev[current_device_slot()];
@@ -801,8 +783,6 @@ int yx_plan_run(yx_plan* p, void* stream, int32_t use_graph) {
     // independent branches (the three head levels) become parallel branches of the graph
     int max_lane = 0;
     for (const auto& o : p->ops) if (o.lane > max_lane) max_lane = o.lane;
-    static const bool lanes_on = !(getenv("YX_LANES") && getenv("YX_LANES")[0] == '0');
-    if (!lanes_on) max_lane = 0;
     while ((int)p->lane_streams.size() < max_lane) {
       cudaStream_t st = nullptr;
       YX_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));

@@ -24,12 +24,6 @@
 
 namespace yx {
 
-#ifdef YX_EXP_BNECK128
-static constexpr bool kHasBneck128 = true;
-#else
-static constexpr bool kHasBneck128 = false;
-#endif
-
 static constexpr int kBnX = 6;          // max X halo slots
 static constexpr int kBnThreads = 64 + 256 + 256 + 32;   // TMA + GEMM2 warps, 8 epilogue-1 warps (4 per GEMM1 tile), 8 epilogue-2 warps, GEMM1 warp
 static constexpr int kWarpG1 = 18;
@@ -46,14 +40,9 @@ struct BneckParams {
   unsigned desc_hi, idesc, tmem_cols, bias_bytes, swz_mask;
   unsigned mul_tpi, mul_tw;
   int act1;
-  int trace;
   const float* bias1;
   EpiParams epi;             // second conv: bias2, act, out, res (= x when the block has a shortcut)
 };
-
-// YX_BNECK_TRACE=1: CTA 0 records clock64() at the hand-off points of its first tiles (diagnostic)
-__device__ long long g_bneck_trace[4][16][4];
-#define BN_TRACE(role, it, k) do { if (p.trace && blockIdx.x == 0 && (it) < 16 && (threadIdx.x & 31) == 0 && ((role) != 1 || warp == 2) && ((role) != 2 || warp == 10 || warp == 14)) g_bneck_trace[role][it][k] = clock64(); } while (0)
 
 struct __align__(8) BneckShared {
   uint64_t xfull[kBnX], xempty[kBnX];
@@ -105,8 +94,8 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
   tc_fence_after();
   // Values every role needs are NOT kept in registers across the role branch: at the 96-register cap of this CTA size ptxas
   // spilled exactly those (tmem_base, tiles per image) to local memory, and with the L1 carved out for shared memory every
-  // reload in the per-tile loops was an L2 round trip (~700 clk per tile in epilogue 1, the critical stage; clock64 trace
-  // with YX_BNECK_TRACE=1). Each role re-reads them from shared memory / the constant bank instead.
+  // reload in the per-tile loops was an L2 round trip (~700 clk per tile in epilogue 1, the critical stage, measured
+  // with a clock64 trace). Each role re-reads them from shared memory / the constant bank instead.
 #define tmem_base (sh->tmem_base)
 #define tiles_per_img (p.tiles_per_img)
   pdl_launch_dependents();      // the weights are constants: loaded before griddepcontrol.wait (see the producer)
@@ -132,7 +121,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
         const int ty = fast_div(r, p.mul_tw, p.tiles_w);
         const int tx = r - ty * p.tiles_w;
         mbar_wait(&sh->xempty[sx], px ^ 1);
-        BN_TRACE(3, t - t_begin, 0);
         mbar_arrive_expect_tx(&sh->xfull[sx], p.x_tx_bytes);
         tma_load_4d(&map_x, &sh->xfull[sx], xs + (size_t)sx * p.x_slot_bytes, 0, tx * p.tw - 1, ty * p.th - 1, b);
         if (++sx == p.nx) { sx = 0; px ^= 1; }
@@ -152,13 +140,10 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
     int sx = 0;
     uint32_t px = 0;
     for (int it = 0; it < n_my; ++it) {
-      BN_TRACE(0, it, 0);
       const int st = it & 1;
       const uint32_t ph = (uint32_t)((it >> 1) & 1);
       mbar_wait(&sh->hfull[st], ph);
-      BN_TRACE(0, it, 1);
       mbar_wait(&sh->a2empty[st], ph ^ 1);
-      BN_TRACE(0, it, 2);
       tc_fence_after();
       if (elect_one_sync()) {
         const uint64_t hd = dhi | (uint64_t)(h16 + (uint32_t)st * hslot16);
@@ -174,7 +159,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
         umma_commit(&sh->hempty[st]);
       }
       __syncwarp();
-      BN_TRACE(0, it, 3);
     }
   } else if (warp == kWarpG1) {
     // ===================== GEMM1 issuer (own warp: its waits and commits never delay GEMM2) =====================
@@ -191,9 +175,7 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
     for (int k = 0; k < n_my; ++k) {
       const int st = k & 1;
       mbar_wait(&sh->xfull[sx], px);
-      BN_TRACE(3, k, 1);
       mbar_wait(&sh->a1empty[st], (uint32_t)(((k >> 1) & 1) ^ 1));
-      BN_TRACE(3, k, 2);
       tc_fence_after();
       if (elect_one_sync()) {
         const uint64_t xd = dhi | (uint64_t)(x16 + (uint32_t)sx * xslot16);
@@ -233,7 +215,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
       const int st = it & 1;
       const uint32_t ph = (uint32_t)((it >> 1) & 1);
       mbar_wait(&sh->a1full[st], ph);
-      BN_TRACE(1, it, 1);
       tc_fence_after();
       // the first TMEM loads are issued before the wait for the hidden-tile slot: that wait (a shared-memory round trip of
       // ~170 clk even when the phase completed long ago) overlaps their latency
@@ -245,7 +226,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
         for (int k = 0; k < KH; ++k) tmem_ld_x16(taddr + (uint32_t)(16 * k), raw[k]);
       }
       mbar_wait(&sh->hempty[st], ph ^ 1);
-      BN_TRACE(1, it, 2);
       uint8_t* hslot = hs + (size_t)st * p.h_slot_bytes;
       if (warp_live) {
         const int iy = ty * p.th - 1 + yy, ix = tx * p.tw - 1 + xx;
@@ -310,12 +290,10 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
           for (int k = 0; k < KH; ++k) emit(raw[k], 16 * (k0 + k));
         }
       }
-      BN_TRACE(1, it, 0);
       tc_fence_before();
       mbar_arrive(&sh->a1empty[st]);
       fence_proxy_async();                     // generic-proxy stores -> visible to the tensor core
       mbar_arrive(&sh->hfull[st]);
-      BN_TRACE(1, it, 3);
     }
   } else {
     // ===================== epilogue 2: y = act(acc2 + b2) (+ x) =====================
@@ -335,9 +313,7 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
       const bool valid = row_ok && ho < p.H && wo < p.W && b < p.batch;
       const long long pix = ((long long)b * p.H + ho) * p.W + wo;
       const int st = it & 1;
-      BN_TRACE(2, it, 0);
       mbar_wait(&sh->a2full[st], (uint32_t)((it >> 1) & 1));
-      BN_TRACE(2, it, 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc2_col + (uint32_t)(st * p.Cpad);
       uint16_t* orow = (uint16_t*)p.epi.out + pix * p.epi.out_ld;
@@ -361,7 +337,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
       }
       tc_fence_before();
       mbar_arrive(&sh->a2empty[st]);
-      BN_TRACE(2, it, 2);
     }
   }
 
@@ -374,300 +349,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
 #undef tmem_base
 #undef tiles_per_img
 }
-
-#ifdef YX_EXP_BNECK128   // negative result (DESIGN 4.6): only in experiment builds (python -m pixeltable_yolox_b200.build --exp -DYX_EXP_BNECK128)
-// ------------------------------------------------------------------------------------------
-// C = 128: two 64-channel chunks, W2 (288 KB) cannot stay resident. Same five steps as above with
-//   * X: one slot of two chunk tiles; H: two slots of two chunk tiles; TMEM: acc1 (2 x 128 columns, single)
-//     + acc2 (2 stages x 128) = 512 columns
-//   * a ring of kB2Stages 16 KB weight stages fed by its own producer warp in the order
-//       W1(0) W1(1) | W2(0) W1(2) | W2(1) W1(3) | ...        (W1(j) = 2 stages, W2(k) = 18 stages, chunk-major)
-//     i.e. the weights of GEMM1(k+2) sit right behind those of GEMM2(k): GEMM1 of the next tile is fed while
-//     GEMM2 of the current one runs, so epilogue 1 of tile k+1 overlaps GEMM2(k) and the tensor core only idles
-//     during the first tile. ONE warp issues both GEMMs in ring order (two issuers at different ring positions would
-//     alias on the parity waits).
-// ------------------------------------------------------------------------------------------
-static constexpr int kB2Stages = 3;
-static constexpr int kB2Threads = 64 + 256 + 256 + 32;        // + weight producer warp (18)
-
-struct __align__(8) Bneck2Shared {
-  uint64_t xfull, xempty;
-  uint64_t a1full, a1empty;
-  uint64_t hfull[2], hempty[2];
-  uint64_t a2full[2], a2empty[2];
-  uint64_t wfull[kB2Stages], wempty[kB2Stages];
-  uint32_t tmem_base;
-};
-
-template <bool FP16, bool SILU>
-__global__ void __launch_bounds__(kB2Threads, 1)
-bneck128_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w1,
-                   const __grid_constant__ CUtensorMap map_w2, const BneckParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  Bneck2Shared* sh = reinterpret_cast<Bneck2Shared*>(smem);
-  float* sbias1 = reinterpret_cast<float*>(smem + 1024);
-  float* sbias2 = sbias1 + p.bias_bytes / 4;
-  constexpr int C = 128, NCH = 2;
-  const uint32_t chunk_bytes = p.x_slot_bytes;                    // one 64-channel halo tile
-  uint8_t* xs = smem + 1024 + 2 * p.bias_bytes;                    // [NCH] halo of x
-  uint8_t* hs = xs + NCH * chunk_bytes;                            // [2][NCH] hidden halo tiles
-  uint8_t* ws = hs + 2 * NCH * chunk_bytes;                        // [kB2Stages] weight stages [128 x 64]
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr bool silu_tanh = SILU && !FP16;
-  {
-    const float s1 = silu_tanh ? 0.5f : 1.0f;
-    for (int i = threadIdx.x; i < C; i += blockDim.x) { sbias1[i] = p.bias1[i] * s1; sbias2[i] = p.epi.bias[i] * s1; }
-  }
-  if (threadIdx.x == 0) {
-    tma_prefetch_desc(&map_x); tma_prefetch_desc(&map_w1); tma_prefetch_desc(&map_w2);
-    mbar_init(&sh->xfull, 1); mbar_init(&sh->xempty, 1);
-    mbar_init(&sh->a1full, 1); mbar_init(&sh->a1empty, 256);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&sh->hfull[i], 256); mbar_init(&sh->hempty[i], 1);
-      mbar_init(&sh->a2full[i], 1); mbar_init(&sh->a2empty[i], 128);
-    }
-    for (int i = 0; i < kB2Stages; ++i) { mbar_init(&sh->wfull[i], 1); mbar_init(&sh->wempty[i], 1); }
-    fence_barrier_init();
-  }
-  if (warp == 1) { tmem_alloc(&sh->tmem_base, 512); tmem_relinquish(); }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = sh->tmem_base;
-  pdl_launch_dependents();
-
-  const int tiles_per_img = p.tiles_w * p.tiles_h;
-  const long long T = p.num_tiles;
-  const int t_begin = (int)(T * blockIdx.x / gridDim.x), t_end = (int)(T * (blockIdx.x + 1) / gridDim.x);
-  const int n_my = t_end - t_begin;
-  const uint32_t acc1_col = 0, acc2_col = 256;
-  const uint64_t dhi = ((uint64_t)p.desc_hi << 32) | (1u << 16);
-  const uint32_t rb16 = 8, prb16 = (uint32_t)p.pitch * 8;        // 128-byte rows
-  const uint32_t ch16 = chunk_bytes >> 4, st16 = 16384u >> 4;
-
-  if (warp == 0) {
-    // ===================== X producer =====================
-    if (lane == 0) {
-      pdl_wait();
-      for (int j = 0; j < n_my; ++j) {
-        const int t = t_begin + j;
-        const int b = fast_div(t, p.mul_tpi, tiles_per_img);
-        const int r = t - b * tiles_per_img;
-        const int ty = fast_div(r, p.mul_tw, p.tiles_w);
-        const int tx = r - ty * p.tiles_w;
-        mbar_wait(&sh->xempty, (uint32_t)((j & 1) ^ 1));
-        mbar_arrive_expect_tx(&sh->xfull, NCH * p.x_tx_bytes);
-        for (int c = 0; c < NCH; ++c)
-          tma_load_4d(&map_x, &sh->xfull, xs + (size_t)c * chunk_bytes, c * 64, tx * p.tw - 1, ty * p.th - 1, b);
-      }
-    }
-  } else if (warp == 18) {
-    // ===================== weight producer: the virtual sequence, one 16 KB stage per entry =====================
-    if (lane == 0) {
-      int pos = 0;
-      auto put = [&](const CUtensorMap* m, int kcoord) {
-        const int stg = pos % kB2Stages;
-        mbar_wait(&sh->wempty[stg], (uint32_t)(((pos / kB2Stages) & 1) ^ 1));
-        mbar_arrive_expect_tx(&sh->wfull[stg], 16384u);
-        tma_load_2d(m, &sh->wfull[stg], ws + (size_t)stg * 16384u, kcoord, 0);
-        ++pos;
-      };
-      auto put_w1 = [&]() { for (int c = 0; c < NCH; ++c) put(&map_w1, c * 64); };
-      if (n_my > 0) put_w1();
-      if (n_my > 1) put_w1();
-      for (int k = 0; k < n_my; ++k) {
-        for (int c = 0; c < NCH; ++c)
-          for (int tap = 0; tap < 9; ++tap) put(&map_w2, tap * C + c * 64);
-        if (k + 2 < n_my) put_w1();
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer: GEMM1 and GEMM2 in the order of the weight ring =====================
-    // One warp walks the virtual sequence, so every wait on wfull[] is for the ring's NEXT phase. (Two issuing warps at
-    // different ring positions alias: a parity wait cannot tell phase q from phase q + 2.)
-    const uint32_t x16 = smem_u32(xs) >> 4, h16 = smem_u32(hs) >> 4, w16 = smem_u32(ws) >> 4;
-    const uint32_t idesc = p.idesc;
-    int pos = 0;
-    auto gemm1 = [&](int j) {
-      mbar_wait(&sh->xfull, (uint32_t)(j & 1));
-      mbar_wait(&sh->a1empty, (uint32_t)((j & 1) ^ 1));
-      tc_fence_after();
-      for (int c = 0; c < NCH; ++c, ++pos) {
-        const int stg = pos % kB2Stages;
-        mbar_wait(&sh->wfull[stg], (uint32_t)((pos / kB2Stages) & 1));
-        tc_fence_after();
-        if (elect_one_sync()) {
-          const uint64_t bd = dhi | (uint64_t)(w16 + (uint32_t)stg * st16);
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt) {
-            const uint64_t ad = dhi | (uint64_t)(x16 + (uint32_t)c * ch16 + (uint32_t)(mt * 128) * rb16);
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-              umma_f16(tmem_base + acc1_col + (uint32_t)(mt * 128), ad + 2 * i, bd + 2 * i, idesc, (uint32_t)((c | i) != 0));
-          }
-          umma_commit(&sh->wempty[stg]);
-        }
-        __syncwarp();
-      }
-      if (elect_one_sync()) { umma_commit(&sh->a1full); umma_commit(&sh->xempty); }
-      __syncwarp();
-    };
-    auto gemm2 = [&](int k) {
-      const int st = k & 1;
-      const uint32_t ph = (uint32_t)((k >> 1) & 1);
-      mbar_wait(&sh->hfull[st], ph);
-      mbar_wait(&sh->a2empty[st], ph ^ 1);
-      tc_fence_after();
-      const uint32_t d2 = tmem_base + acc2_col + (uint32_t)(st * 128);
-      for (int c = 0; c < NCH; ++c) {
-#pragma unroll
-        for (int tap = 0; tap < 9; ++tap, ++pos) {
-          const int stg = pos % kB2Stages;
-          mbar_wait(&sh->wfull[stg], (uint32_t)((pos / kB2Stages) & 1));
-          tc_fence_after();
-          if (elect_one_sync()) {
-            const uint64_t bd = dhi | (uint64_t)(w16 + (uint32_t)stg * st16);
-            const uint64_t ad = dhi | (uint64_t)(h16 + (uint32_t)(st * NCH + c) * ch16 + (uint32_t)(tap / 3) * prb16 + (uint32_t)(tap % 3) * rb16);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) umma_f16(d2, ad + 2 * i, bd + 2 * i, idesc, (uint32_t)((c | tap | i) != 0));
-            umma_commit(&sh->wempty[stg]);
-          }
-          __syncwarp();
-        }
-      }
-      if (elect_one_sync()) { umma_commit(&sh->a2full[st]); umma_commit(&sh->hempty[st]); }
-      __syncwarp();
-    };
-    if (n_my > 0) gemm1(0);
-    if (n_my > 1) gemm1(1);
-    for (int k = 0; k < n_my; ++k) {
-      gemm2(k);
-      if (k + 2 < n_my) gemm1(k + 2);
-    }
-  } else if (warp < 10) {
-    // ===================== epilogue 1 (warps 2..5: halo rows 0..127, warps 6..9: rows 128..) =====================
-    const int quarter = warp & 3;
-    const int t128 = quarter * 32 + lane;
-    const int mt = (warp - 2) >> 2;
-    const int q = mt * 128 + t128;
-    const int yy = q / p.pitch, xx = q - yy * p.pitch;
-    const bool warp_live = mt * 128 + quarter * 32 < p.halo_rows + 2;
-    const bool stored = q < p.halo_rows + 2;
-    const uint32_t rowoff = (uint32_t)q * 128u;
-    const uint32_t xr = (uint32_t)q & 7u;
-    for (int k = 0; k < n_my; ++k) {
-      const int t = t_begin + k;
-      const int b = fast_div(t, p.mul_tpi, tiles_per_img);
-      const int r = t - b * tiles_per_img;
-      const int ty = fast_div(r, p.mul_tw, p.tiles_w);
-      const int tx = r - ty * p.tiles_w;
-      const int st = k & 1;
-      mbar_wait(&sh->a1full, (uint32_t)(k & 1));
-      mbar_wait(&sh->hempty[st], (uint32_t)(((k >> 1) & 1) ^ 1));
-      tc_fence_after();
-      if (warp_live) {
-        const int iy = ty * p.th - 1 + yy, ix = tx * p.tw - 1 + xx;
-        const bool inside = (q < p.halo_rows) && iy >= 0 && iy < p.H && ix >= 0 && ix < p.W && b < p.batch;
-        const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc1_col + (uint32_t)(mt * 128);
-#pragma unroll
-        for (int c = 0; c < NCH; ++c) {
-          uint8_t* hchunk = hs + (size_t)(st * NCH + c) * chunk_bytes + rowoff;
-          uint32_t raw[4][16];
-#pragma unroll
-          for (int g = 0; g < 4; ++g) tmem_ld_x16(taddr + (uint32_t)(c * 64 + g * 16), raw[g]);
-          tmem_ld_wait();
-#pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            uint32_t w[8];
-            if (inside) {
-              float v[16];
-#pragma unroll
-              for (int j = 0; j < 16; j += 4) {
-                const float4 bb = *reinterpret_cast<const float4*>(sbias1 + c * 64 + g * 16 + j);
-                const float hb[4] = {bb.x, bb.y, bb.z, bb.w};
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                  if constexpr (silu_tanh) {
-                    const float h = fmaf(__uint_as_float(raw[g][j + u]), 0.5f, hb[u]);
-                    float tt;
-                    asm("tanh.approx.f32 %0, %1;" : "=f"(tt) : "f"(h));
-                    v[j + u] = fmaf(h, tt, h);
-                  } else if constexpr (SILU && FP16) {
-                    v[j + u] = silu_exp(__uint_as_float(raw[g][j + u]) + hb[u]);
-                  } else {
-                    v[j + u] = act_f<false>(__uint_as_float(raw[g][j + u]) + hb[u], p.act1);
-                  }
-                }
-              }
-#pragma unroll
-              for (int j = 0; j < 8; ++j) w[j] = pack16_t<FP16>(v[2 * j], v[2 * j + 1]);
-            } else {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) w[j] = 0u;
-            }
-            if (stored) {
-              *reinterpret_cast<uint4*>(hchunk + ((((uint32_t)(2 * g)) ^ xr) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
-              *reinterpret_cast<uint4*>(hchunk + ((((uint32_t)(2 * g + 1)) ^ xr) << 4)) = make_uint4(w[4], w[5], w[6], w[7]);
-            }
-          }
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(&sh->a1empty);
-      fence_proxy_async();
-      mbar_arrive(&sh->hfull[st]);
-    }
-  } else if (warp < 18) {
-    // ===================== epilogue 2 =====================
-    pdl_wait();
-    const int quarter = warp & 3;
-    const int row = quarter * 32 + lane;
-    const int hl0 = row / p.pitch, wl0 = row - hl0 * p.pitch;
-    const bool row_ok = hl0 < p.th && wl0 < p.tw;
-    const int grp = (warp - 10) >> 2;
-    for (int k = grp; k < n_my; k += 2) {
-      const int t = t_begin + k;
-      const int b = fast_div(t, p.mul_tpi, tiles_per_img);
-      const int r = t - b * tiles_per_img;
-      const int ty = fast_div(r, p.mul_tw, p.tiles_w);
-      const int tx = r - ty * p.tiles_w;
-      const int ho = ty * p.th + hl0, wo = tx * p.tw + wl0;
-      const bool valid = row_ok && ho < p.H && wo < p.W && b < p.batch;
-      const long long pix = ((long long)b * p.H + ho) * p.W + wo;
-      const int st = k & 1;
-      mbar_wait(&sh->a2full[st], (uint32_t)((k >> 1) & 1));
-      tc_fence_after();
-      const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc2_col + (uint32_t)(st * 128);
-      uint16_t* orow = (uint16_t*)p.epi.out + pix * p.epi.out_ld;
-      const uint16_t* rrow = p.epi.res ? (const uint16_t*)p.epi.res + pix * p.epi.res_ld : nullptr;
-#pragma unroll
-      for (int c = 0; c < C; c += 32) {
-        uint32_t ra[16], rb[16];
-        tmem_ld_x16(taddr + (uint32_t)c, ra);
-        tmem_ld_x16(taddr + (uint32_t)(c + 16), rb);
-        uint32_t qa[8], qb[8];
-        if (rrow && valid) { ld_global_256(rrow + c, qa); ld_global_256(rrow + c + 16, qb); }
-        tmem_ld_wait();
-        if (valid) {
-          epi_tc_chunk<FP16, SILU>(p.epi, ra, sbias2 + c, rrow ? qa : nullptr, orow + c, b, ho, wo, c);
-          epi_tc_chunk<FP16, SILU>(p.epi, rb, sbias2 + c + 16, rrow ? qb : nullptr, orow + c + 16, b, ho, wo, c + 16);
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(&sh->a2empty[st]);
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-#endif  // YX_EXP_BNECK128
 
 // ------------------------------------------------------------------------------------------
 // host side
@@ -694,12 +375,12 @@ BneckLaunch* bneck_alloc() {
 void bneck_free(BneckLaunch* p) { free(p); }
 
 bool bneck_supported(const yx_bneck_desc* d) {
-  return d && (d->c == 16 || d->c == 32 || d->c == 64 || (kHasBneck128 && d->c == 128)) && (d->dtype == YX_BF16 || d->dtype == YX_FP16);
+  return d && (d->c == 16 || d->c == 32 || d->c == 64) && (d->dtype == YX_BF16 || d->dtype == YX_FP16);
 }
 
 int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
   YX_REQUIRE(d != nullptr, YX_ERR_INVALID_ARG, "bottleneck: null descriptor");
-  YX_REQUIRE(d->c == 16 || d->c == 32 || d->c == 64 || (kHasBneck128 && d->c == 128), YX_ERR_UNSUPPORTED, "bottleneck: c=%d (fused kernel: 16, 32 or 64)", d->c);
+  YX_REQUIRE(d->c == 16 || d->c == 32 || d->c == 64, YX_ERR_UNSUPPORTED, "bottleneck: c=%d (fused kernel: 16, 32 or 64)", d->c);
   YX_REQUIRE(d->dtype == YX_BF16 || d->dtype == YX_FP16, YX_ERR_INVALID_ARG, "bottleneck: dtype must be bf16/fp16");
   YX_REQUIRE(d->batch > 0 && d->h > 0 && d->w > 0, YX_ERR_INVALID_ARG, "bottleneck: empty input");
   YX_REQUIRE(d->x && d->w1 && d->w2 && d->bias1 && d->bias2 && d->out, YX_ERR_INVALID_ARG, "bottleneck: null pointer");
@@ -730,10 +411,8 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
   p.C = d->c; p.Cpad = d->c < 32 ? 32 : d->c;
   p.batch = d->batch; p.H = d->h; p.W = d->w;
   p.ksteps = d->c / 16;
-  const bool big = d->c == 128;                            // two 64-channel chunks, streamed weights (bneck128_tc_kernel)
-  const int kc = big ? 64 : d->c;                           // channels per shared-memory row
-  p.row_bytes = (unsigned)kc * 2u;
-  p.swz_mask = kc == 64 ? 7u : (kc == 32 ? 3u : 1u);
+  p.row_bytes = (unsigned)d->c * 2u;
+  p.swz_mask = d->c == 64 ? 7u : (d->c == 32 ? 3u : 1u);
   long long best = -1; int btw = 1, bth = 1;
   for (int tw = 1; tw <= d->w && tw + 2 <= 128; ++tw) {
     int th = 128 / (tw + 2);
@@ -743,10 +422,6 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
     const long long tiles = ceil_div64(d->w, tw) * ceil_div64(d->h, th);
     const long long cost = tiles * 4096 + (long long)(th + 2) * (tw + 2);
     if (best < 0 || cost < best) { best = cost; btw = tw; bth = th; }
-  }
-  if (const char* e = getenv("YX_BN_TW")) {          // experiment: force the tile width
-    const int tw = atoi(e);
-    if (tw >= 1 && tw + 2 <= 128) { btw = tw < d->w ? tw : d->w; bth = 128 / (btw + 2); if (bth > d->h) bth = d->h; }
   }
   p.tw = btw; p.th = bth; p.pitch = btw + 2;
   p.halo_rows = (p.th + 2) * p.pitch;
@@ -760,16 +435,15 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
   p.x_slot_bytes = ((unsigned)(p.halo_rows + 2) * p.row_bytes + 1023u) & ~1023u;
   p.h_slot_bytes = p.x_slot_bytes;
   p.x_tx_bytes = (unsigned)p.halo_rows * p.row_bytes;
-  p.w_tile_bytes = ((unsigned)d->c * p.row_bytes + 1023u) & ~1023u;   // [N = c rows x kc channels]
+  p.w_tile_bytes = ((unsigned)d->c * p.row_bytes + 1023u) & ~1023u;   // [N = c rows x c channels]
   p.w_tx_bytes = (unsigned)d->c * p.row_bytes;
   p.bias_bytes = 1024u;
   p.tmem_cols = 32; while (p.tmem_cols < (unsigned)(6 * p.Cpad)) p.tmem_cols <<= 1;
-  const unsigned layout = kc == 64 ? 2u : (kc == 32 ? 4u : 6u);
+  const unsigned layout = d->c == 64 ? 2u : (d->c == 32 ? 4u : 6u);
   p.desc_hi = (((8u * p.row_bytes) >> 4) & 0x3FFFu) | (1u << 14) | (layout << 29);
   const unsigned fmt = d->dtype == YX_BF16 ? 1u : 0u;
   p.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((unsigned)(d->c >> 3) << 17) | ((128u >> 4) << 24);
   p.act1 = d->act; p.bias1 = d->bias1;
-  p.trace = getenv("YX_BNECK_TRACE") ? 1 : 0;
   EpiParams& e = p.epi;
   e.out_h = d->h; e.out_w = d->w; e.out_c = d->c; e.act = d->act; e.dtype = d->dtype; e.epilogue = YX_EPI_STORE;
   e.bias = d->bias2; e.out = d->out; e.out_ld = d->out_ld;
@@ -778,23 +452,17 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
   YX_CUDA(cudaGetDevice(&dev));
   YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
   const long long fixed = 2048 + 2 * (long long)p.bias_bytes + 2 * (long long)p.h_slot_bytes + 10 * (long long)p.w_tile_bytes;
-  if (big) {
-    p.nx = 1;
-    L->smem = 2048 + 2 * (size_t)p.bias_bytes + 6 * (size_t)p.x_slot_bytes + 3 * 16384;
-    YX_REQUIRE((long long)L->smem <= max_smem, YX_ERR_UNSUPPORTED, "bottleneck(128): needs %zu bytes of shared memory", L->smem);
-  } else {
-    p.nx = (int)((max_smem - fixed) / p.x_slot_bytes);
-    if (p.nx > kBnX) p.nx = kBnX;
-    YX_REQUIRE(p.nx >= 2, YX_ERR_UNSUPPORTED, "bottleneck: shared memory too small (%lld fixed bytes)", fixed);
-    L->smem = (size_t)fixed + (size_t)p.nx * p.x_slot_bytes;
-  }
+  p.nx = (int)((max_smem - fixed) / p.x_slot_bytes);
+  if (p.nx > kBnX) p.nx = kBnX;
+  YX_REQUIRE(p.nx >= 2, YX_ERR_UNSUPPORTED, "bottleneck: shared memory too small (%lld fixed bytes)", fixed);
+  L->smem = (size_t)fixed + (size_t)p.nx * p.x_slot_bytes;
 
   const CUtensorMapDataType tdt = d->dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  const CUtensorMapSwizzle sw = kc == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (kc == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+  const CUtensorMapSwizzle sw = d->c == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (d->c == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
   {
     cuuint64_t dims[4] = {(cuuint64_t)d->c, (cuuint64_t)d->w, (cuuint64_t)d->h, (cuuint64_t)d->batch};
     cuuint64_t strides[3] = {(cuuint64_t)d->x_ld * 2, (cuuint64_t)d->x_ld * 2 * d->w, (cuuint64_t)d->x_ld * 2 * d->w * d->h};
-    cuuint32_t box[4] = {(cuuint32_t)kc, (cuuint32_t)p.pitch, (cuuint32_t)(p.th + 2), 1};
+    cuuint32_t box[4] = {(cuuint32_t)d->c, (cuuint32_t)p.pitch, (cuuint32_t)(p.th + 2), 1};
     cuuint32_t estr[4] = {1, 1, 1, 1};
     CUresult r = encode(&L->map_x, tdt, 4, const_cast<void*>(d->x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -804,7 +472,7 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
     const cuuint64_t K = (cuuint64_t)(which ? 9 : 1) * d->c;
     cuuint64_t dims[2] = {K, (cuuint64_t)d->c};
     cuuint64_t strides[1] = {K * 2};
-    cuuint32_t box[2] = {(cuuint32_t)kc, (cuuint32_t)d->c};
+    cuuint32_t box[2] = {(cuuint32_t)d->c, (cuuint32_t)d->c};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = encode(which ? &L->map_w2 : &L->map_w1, tdt, 2, const_cast<void*>(which ? d->w2 : d->w1), dims, strides, box, estr,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -826,62 +494,26 @@ int bneck_launch(const BneckLaunch* L, cudaStream_t stream) {
   YX_CUDA(cudaFuncSetAttribute(bneck_tc_kernel<F, K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem))
     YX_BN_ATTR(false, 1); YX_BN_ATTR(false, 2); YX_BN_ATTR(false, 4); YX_BN_ATTR(true, 1); YX_BN_ATTR(true, 2); YX_BN_ATTR(true, 4);
 #undef YX_BN_ATTR
-#ifdef YX_EXP_BNECK128
-#define YX_B2_ATTR(F, S) YX_CUDA(cudaFuncSetAttribute(bneck128_tc_kernel<F, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem))
-    YX_B2_ATTR(false, false); YX_B2_ATTR(false, true); YX_B2_ATTR(true, false); YX_B2_ATTR(true, true);
-#undef YX_B2_ATTR
-#endif
     attr_set = true;
   }
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)L->grid);
-  cfg.blockDim = dim3((unsigned)(L->p.C == 128 ? 64 + 256 + 256 + 32 : kBnThreads));
+  cfg.blockDim = dim3((unsigned)kBnThreads);
   cfg.dynamicSmemBytes = L->smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   const bool h16 = L->p.epi.dtype == YX_FP16;
-#ifdef YX_EXP_BNECK128
-  if (L->p.C == 128) {
-    const bool silu = L->p.act1 == YX_ACT_SILU;
-    if (L->p.trace) { int z[8] = {0, 0, 0, 0, 0, 0, 0, 1}; YX_CUDA(cudaMemcpyToSymbol(g_mbar_dbg, z, sizeof(z))); }
-#define YX_B2_GO(F, S) YX_CUDA(cudaLaunchKernelEx(&cfg, bneck128_tc_kernel<F, S>, L->map_x, L->map_w1, L->map_w2, L->p))
-    if (h16) { if (silu) YX_B2_GO(true, true); else YX_B2_GO(true, false); }
-    else { if (silu) YX_B2_GO(false, true); else YX_B2_GO(false, false); }
-#undef YX_B2_GO
-    if (L->p.trace) {
-      int z[8];
-      cudaError_t e = cudaStreamSynchronize(stream);
-      fprintf(stderr, "bneck128: sync -> %s\n", cudaGetErrorString(e));
-      if (cudaMemcpyFromSymbol(z, g_mbar_dbg, sizeof(z)) == cudaSuccess)
-        fprintf(stderr, "bneck128: mbar timeout=%d block=%d thread=%d (warp %d) bar_smem=0x%x parity=%d\n", z[0], z[1], z[2], z[2] / 32, z[3], z[4]);
-    }
-    return YX_OK;
-  }
-#endif
 #define YX_BN_GO(F, K) do { if (L->p.act1 == YX_ACT_SILU) YX_CUDA(cudaLaunchKernelEx(&cfg, bneck_tc_kernel<F, K, true>, L->map_x, L->map_w1, L->map_w2, L->p)); \
     else YX_CUDA(cudaLaunchKernelEx(&cfg, bneck_tc_kernel<F, K, false>, L->map_x, L->map_w1, L->map_w2, L->p)); } while (0)
   if (L->p.ksteps == 4) { if (h16) YX_BN_GO(true, 4); else YX_BN_GO(false, 4); }
   else if (L->p.ksteps == 2) { if (h16) YX_BN_GO(true, 2); else YX_BN_GO(false, 2); }
   else { if (h16) YX_BN_GO(true, 1); else YX_BN_GO(false, 1); }
 #undef YX_BN_GO
-  if (L->p.trace) {
-    long long h[4][16][4];
-    YX_CUDA(cudaStreamSynchronize(stream));
-    YX_CUDA(cudaMemcpyFromSymbol(h, g_bneck_trace, sizeof(h)));
-    const long long t0 = h[3][0][0];
-    const char* names[4] = {"mma : g1(next) issued | hfull seen | a2empty seen | g2 issued", "epi1: stores issued | a1full seen | hempty seen | done",
-                            "epi2: start | a2full seen | done", "tma : xempty seen | (mma) xfull seen | (mma) a1empty seen"};
-    for (int r = 0; r < 4; ++r) {
-      fprintf(stderr, "%s\n", names[r]);
-      for (int i = 0; i < 12; ++i)
-        fprintf(stderr, "  tile %2d: %8lld %8lld %8lld %8lld\n", i, h[r][i][0] - t0, h[r][i][1] - t0, h[r][i][2] - t0, h[r][i][3] - t0);
-    }
-  }
   return YX_OK;
 }
 

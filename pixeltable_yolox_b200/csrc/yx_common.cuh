@@ -42,26 +42,17 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
   } while (0)
 
 int num_sms();  // SM count of the current device (cached)
-bool pdl_enabled();  // programmatic dependent launch between consecutive plan kernels (YX_PDL=0 disables)
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline int dtype_size(int dt) { return dt == YX_FP32 ? 4 : (dt == YX_U8 ? 1 : 2); }
 
 #ifdef __CUDACC__
-// Launch with programmatic stream serialization: the kernel may start while its predecessor drains, provided the predecessor
-// called griddepcontrol.launch_dependents; the kernel itself must execute griddepcontrol.wait (pdl_wait) before it touches
-// memory. For the training step's chains of small kernels (BatchNorm, wgrad, packing) this measured SLOWER than plain
-// launches (9.32 vs 8.70 ms per step, 8 images): off unless YX_TRAIN_PDL=1.
-bool train_pdl_enabled();
+// Plain launch that returns the launch error. The training step's chains of small kernels (BatchNorm, wgrad, packing) do
+// not use programmatic dependent launch: it measured slower than plain launches there (9.32 vs 8.70 ms per step, 8 images).
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
+inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = train_pdl_enabled() ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
@@ -123,30 +114,16 @@ __device__ __forceinline__ uint32_t orderable_f32(float f) {
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 // Bounded spin: a pipeline bug must surface as a trapped launch, never as a hung GPU.
-// g_mbar_dbg (one copy per translation unit): [0] timeout seen, [1..4] block / thread / barrier smem address / parity of
-// the first one, [7] != 0: do not trap, give up the wait instead (diagnostic runs read the record back afterwards).
-static __device__ int g_mbar_dbg[8];
-// cold path, kept out of line so the waiting loops stay a handful of instructions; returns true to give up the wait
-static __device__ __noinline__ bool mbar_timed_out(uint32_t bar_smem, uint32_t parity) {
-  if (atomicCAS(&g_mbar_dbg[0], 0, 1) == 0) {
-    g_mbar_dbg[1] = (int)blockIdx.x; g_mbar_dbg[2] = (int)threadIdx.x;
-    g_mbar_dbg[3] = (int)bar_smem; g_mbar_dbg[4] = (int)parity;
-  }
-  if (g_mbar_dbg[7]) {
-    if ((threadIdx.x & 31) == 0 && blockIdx.x == (unsigned)g_mbar_dbg[1])
-      printf("yx_b200: [no-trap] wait gave up: block %d warp %d barrier smem 0x%x parity %u\n", (int)blockIdx.x, (int)(threadIdx.x >> 5), bar_smem, parity);
-    return true;
-  }
-  printf("yx_b200: mbarrier wait timed out (block %d thread %d parity %u)\n", (int)blockIdx.x, (int)threadIdx.x, parity);
+// cold path, kept out of line so the waiting loops stay a handful of instructions
+static __device__ __noinline__ void mbar_timed_out(uint32_t bar_smem, uint32_t parity) {
+  printf("yx_b200: mbarrier wait timed out (block %d thread %d barrier smem 0x%x parity %u)\n", (int)blockIdx.x,
+         (int)threadIdx.x, bar_smem, parity);
   __trap();
-  return true;
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   uint32_t spins = 0;
   while (!mbar_try_wait(bar, parity)) {
-    if (++spins > (1u << 18)) {
-      if (mbar_timed_out(smem_u32(bar), parity)) return;
-    }
+    if (++spins > (1u << 18)) mbar_timed_out(smem_u32(bar), parity);
   }
 }
 

@@ -60,8 +60,6 @@ struct ConvTcParams {
   unsigned a_slot_bytes, a_tx_bytes, row_bytes;
   int b_resident;        // all 9*kchunks weight tiles stay in smem (n_tiles == 1)
   unsigned b_tile_bytes, b_tx_bytes, b_region_bytes;
-  int pdl_late;          // 1: weights are prefetched before griddepcontrol.wait
-  int base_off;          // 1: set the descriptor base-offset field from the shifted start address
   unsigned mul_tpi, mul_tw, mul_ntiles, mul_ohw, mul_ow;   // floor(2^32 / d) + 1 for tiles_per_img, tiles_w, n_tiles, out_h*out_w, out_w
   // ---- halo == 2 (3x3 stride 2): input viewed as [2C, W/2, H, B] (x parity folded into the channels), one
   //      halo tile per (channel chunk, y parity) "plane kind"; each kind runs a short list of MMA ops
@@ -144,19 +142,6 @@ __device__ __forceinline__ void halo_issue_ring(TcShared* sh, uint64_t ad0, uint
 
 
 // SILU: the activation is SiLU (compile-time: the generic activation code and its per-chunk dispatch disappear)
-// -DYX_CONV_TRACE (experiment builds only, see build.py --exp): CTA 0 records %globaltimer at the hand-off points of its
-// first and last tile; conv_tc_launch prints them. Compiled out of the product library (the hot loops are sensitive to
-// any extra code: see DESIGN 4.4/4.5).
-#ifdef YX_CONV_TRACE
-__device__ unsigned long long g_conv_trace[16];
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define CT(k) do { if (blockIdx.x == 0) g_conv_trace[k] = gtimer(); } while (0)
-#define CT_ONCE(k, flag) do { if (blockIdx.x == 0 && !(flag)) { g_conv_trace[k] = gtimer(); flag = true; } } while (0)
-#else
-#define CT(k) do { } while (0)
-#define CT_ONCE(k, flag) do { } while (0)
-#endif
-
 // HEAD: the YX_EPI_HEAD epilogue (decode + optional score filter) is its own instantiation, so its ~1 000 SASS
 // instructions do not sit in the instruction cache footprint / register allocation of the activation-store kernels
 template <bool FP16, bool SILU, bool HEAD>
@@ -164,7 +149,6 @@ __global__ void __launch_bounds__(kMaxThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                const ConvTcParams p) {
   extern __shared__ uint8_t smem_raw[];
-  if (threadIdx.x == 0) CT(0);
   // operand tiles need 1024-byte alignment for the 128-byte swizzle atom
   // pointer arithmetic on the __shared__ array (not an integer round trip) keeps the address space known to the
   // compiler: LDS/STS instead of generic loads for every bias / staging access
@@ -212,13 +196,11 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = sh->tmem_base;
-  if (threadIdx.x == 0) CT(1);
   // PDL: everything above (barrier init, TMEM allocation, descriptor prefetch, bias copy) touches only
   // constants and overlaps the tail of the previous kernel; activations are read/written after the wait
   // resident weights are constants: their loads are issued BEFORE griddepcontrol.wait (each role waits itself,
   // right before its first access to activations), so they overlap the previous kernel's tail as well
   pdl_launch_dependents();
-  if (p.pdl_late == 0) pdl_wait();   // YX_PDL_EARLY=0: every thread waits here (A/B switch)
 
   const int num_k = p.ksize * p.ksize * p.kchunks;
   const int tiles_per_img = p.tiles_w * p.tiles_h;
@@ -342,10 +324,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                         tap * p.in_c + c * p.KC, 0);
       }
       pdl_wait();
-      CT(2);
       int ca = 0, sb = 0;
       uint32_t pb = 0;
-      [[maybe_unused]] bool tr3 = false;
       for (int t = t_begin; t < t_end;) {
         const int i0 = t % p.G;
         const int u = t / p.G;
@@ -368,7 +348,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             else
               tma_load_4d(&map_a, &sh->afull[slot], aregion + (size_t)slot * p.a_slot_bytes, c * p.KC,
                           tx * p.tw - 1, ty * p.th - 1, b);
-            CT_ONCE(3, tr3);
           }
           if (!p.b_resident) {
             for (int tap = 0; tap < p.taps; ++tap) {
@@ -399,8 +378,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     int sa = 0, sb = 0, as = 0, i0 = t_begin % G;
     uint32_t pa = 0, pb = 0, pacc = 0;
     if (!ring) mbar_wait(&sh->bres_full, 0);
-    if (lane == 0) CT(4);
-    [[maybe_unused]] bool tr5 = false, tr6 = false;
     for (int t = t_begin; t < t_end;) {
       int g = G - i0;
       if (g > t_end - t) g = t_end - t;
@@ -421,7 +398,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       for (int c = 0; c < kch; ++c) {
         const int sl0 = sa;
         mbar_wait(&sh->afull[sa], pa);
-        if (lane == 0) CT_ONCE(5, tr5);
         const uint32_t al0 = a0 + (uint32_t)sa * aslot16;
         if (++sa == n_as) { sa = 0; pa ^= 1; }
         const int sl1 = sa;
@@ -460,7 +436,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         if (g > 1) umma_commit(&sh->tmem_full[st1]);
       }
       __syncwarp();
-      if (lane == 0) CT_ONCE(6, tr6);
       t += g;
     }
   } else if (warp == 0) {
@@ -546,7 +521,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const bool need_coords = (p.flat && (p.epi.ups != nullptr || HEAD)) || p.epi.shuf_c != 0;
     int as = grp % p.acc_stages;
     uint32_t aphase = (uint32_t)((grp / p.acc_stages) & 1);
-    [[maybe_unused]] bool tr7 = false, tr8 = false;
     for (int it = grp;; it += p.epi_groups) {
       int n_tile, m_tile;
       if (p.halo) {
@@ -586,7 +560,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         pix = ((long long)b * p.epi.out_h + ho) * p.epi.out_w + wo;
       }
       mbar_wait(&sh->tmem_full[as], aphase);
-      if (warp == 2 && lane == 0) CT_ONCE(7, tr7);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(as * p.BNpad);
       const float* tbias = sbias + n_tile * p.BN;
@@ -792,7 +765,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       }
       tc_fence_before();
       mbar_arrive(&sh->tmem_empty[as]);
-      if (warp == 2 && lane == 0) { CT_ONCE(8, tr8); CT(9); }
       as += p.epi_groups;
       while (as >= p.acc_stages) { as -= p.acc_stages; aphase ^= 1; }
       }   // !HEAD
@@ -801,7 +773,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) CT(10);
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc(tmem_base, p.tmem_cols);
@@ -907,16 +878,15 @@ int validate_conv_geometry(const yx_conv_desc* d) {
   return YX_OK;
 }
 
-// CTAs per SM for this layer. Measured on the yolox_s step (B = 64, tools/gpu_ctas_experiment.sh, us per launch, 1 -> 2 CTAs):
+// CTAs per SM for this layer. Measured on the yolox_s step (B = 64, us per launch, 1 -> 2 CTAs):
 // two co-resident CTAs pay off where a tile is a handful of MMAs followed by a long epilogue and the single CTA's pipeline
 // is latency-bound -- the stride-2 plane layers with few input channels (32->64 @160: 142 -> 117, 64->128 @80: 78 -> 74) and
 // the 3x3 layers on the 20x20 maps (256->256: 43 -> 39, 128->256: 29 -> 27). They lose where one CTA already keeps the
 // tensor pipe busy (head 3x3 @80x80: 178 -> 203, 3x3 128->128 @40x40: 37 -> 41) or where halving the shared memory evicts the
-// resident weights (1x1 1024->512: 31 -> 37). YX_CTAS_PER_SM=1|2 forces a setting, YX_CTAS_MAXPIX=<pixels> selects by map size.
+// resident weights (1x1 1024->512: 31 -> 37). YX_CTAS_PER_SM=1|2 forces a setting (a test hook).
 static int conv_ctas_per_sm(const yx_conv_desc* d) {
   if (d->epilogue == YX_EPI_HEAD) return 1;                   // the head staging slabs need the shared memory
   if (const char* e = getenv("YX_CTAS_PER_SM")) { const int v = atoi(e); if (v == 1 || v == 2) return v; }
-  if (const char* e = getenv("YX_CTAS_MAXPIX")) return (long long)d->out_h * d->out_w <= atoll(e) ? 2 : 1;
   if (d->ksize == 3 && d->stride == 2 && d->in_c <= 64) return 2;
   if (d->ksize == 3 && d->stride == 1 && d->out_h * d->out_w <= 400 && d->in_c >= 128) return 2;
   return 1;
@@ -972,12 +942,10 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   p.flat = (d->ksize == 1 && d->stride == 1) ? 1 : 0;
   p.halo = (d->ksize == 3 && d->stride == 1) ? 1 : 0;
   p.taps = p.flat ? 1 : 9;
-  if (p.flat && allow_flat) { p.halo = 1; if (const char* e = getenv("YX_HALO_FLAT")) { if (e[0] == '0') p.halo = 0; } }
+  if (p.flat && allow_flat) p.halo = 1;
   // stride 2: the x parity folds into the channel dimension only when pixel pairs are contiguous
   if (allow_s2 && d->ksize == 3 && d->stride == 2 && d->in_ld == d->in_c && d->in_w % 2 == 0 && (d->in_c == 32 || d->in_c % 64 == 0))
     p.halo = 2;
-  if (const char* e = getenv("YX_HALO")) { if (e[0] == '0') p.halo = 0; }
-  if (const char* e = getenv("YX_HALO_S2")) { if (e[0] == '0' && p.halo == 2) p.halo = 0; }
   if (p.halo == 2) { p.KC = 64; p.kchunks = 2 * d->in_c / 64; }
   const unsigned row_bytes = (unsigned)p.KC * 2;             // 128 / 64 / 32 = swizzle span
   p.row_bytes = row_bytes;
@@ -1019,7 +987,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
     // short K loops are epilogue-bound: three tiles in the epilogue at once (MMA cycles per tile ~ k-steps * N / 2)
     p.epi_groups = (p.taps * p.kchunks * (p.KC / 16) * d->out_c <= 4096 && d->out_c <= 128) ? 3 : 2;
     if (d->epilogue == YX_EPI_HEAD) p.epi_groups = 2;                            // staging slabs are 10.9 KB per warp
-    if (const char* e = getenv("YX_EPI_GROUPS")) { int v = atoi(e); if (v >= 1 && v <= kMaxEpiGroups) p.epi_groups = v; }
     YX_REQUIRE(d->epilogue == YX_EPI_STORE || p.flat, YX_ERR_UNSUPPORTED, "conv_tc: the head epilogue needs a 1x1 conv");
     p.head_bytes = d->epilogue == YX_EPI_HEAD ? (((unsigned)p.epi_groups * 4u * 32u * (unsigned)(5 + d->head_nc) * 4u + 1023u) & ~1023u) : 0u;
     const unsigned fixed_bytes = 2048u + p.bias_bytes + p.head_bytes;
@@ -1066,15 +1033,14 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
       p.b_tx_bytes = (unsigned)p.BN * row_bytes;
       b_all = n_btiles * p.b_tile_bytes;
       p.b_resident = (p.n_tiles == 1 && avail - b_all >= 3ll * p.a_slot_bytes) ? 1 : 0;
-      if (const char* e = getenv("YX_HALO_BRES")) { if (e[0] == '0') p.b_resident = 0; }
       if (p.b_resident) break;
     }
     if (p.epi_groups > p.acc_stages) p.epi_groups = p.acc_stages;
     if (ctas == 2) p.epi_groups = 1;
     // stride-2 planes only pay off with resident weights (streamed weights are not shared between M tiles there)
-    if (p.halo == 2 && !p.b_resident && !getenv("YX_HALO_BRES")) return conv_tc_prepare_mode(d, L, false);
+    if (p.halo == 2 && !p.b_resident) return conv_tc_prepare_mode(d, L, false);
     // 1x1 with weights too large to stay resident: the per-tap ring with N up to 256 streams fewer bytes
-    if (p.flat && !p.b_resident && !getenv("YX_HALO_BRES")) return conv_tc_prepare_mode(d, L, allow_s2, false);
+    if (p.flat && !p.b_resident) return conv_tc_prepare_mode(d, L, allow_s2, false);
     if (p.b_resident) {
       p.G = 1;
       p.b_region_bytes = (unsigned)b_all;
@@ -1082,7 +1048,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
       p.a_slots = (int)((avail - b_all) / p.a_slot_bytes);
     } else {
       p.G = (p.acc_stages >= 4 && p.halo == 1) ? 2 : 1;
-      if (p.halo == 1) if (const char* e = getenv("YX_HALO_G")) { int v = atoi(e); if (v >= 1 && v <= 2 && 2 * v <= p.acc_stages) p.G = v; }
       p.a_slots = 2 * p.G;
       long long rest = avail - (long long)p.a_slots * p.a_slot_bytes;
       YX_REQUIRE(rest >= 2ll * p.b_tile_bytes, YX_ERR_UNSUPPORTED, "conv_tc(halo): shared memory too small");
@@ -1097,8 +1062,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
     YX_REQUIRE(p.a_slots >= p.G, YX_ERR_UNSUPPORTED, "conv_tc(halo): halo ring does not fit shared memory");
     const int m_pad = (int)ceil_div64(p.m_tiles, p.G) * p.G;
     p.num_tiles = m_pad * p.n_tiles;
-    p.base_off = 0;
-    if (const char* e = getenv("YX_HALO_BASEOFF")) p.base_off = atoi(e);
     L->smem = fixed_bytes + p.b_region_bytes + (size_t)p.a_slots * p.a_slot_bytes;
   } else {
   if (p.flat) {
@@ -1108,8 +1071,7 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   } else {
     // choose the spatial tile (tw x th <= 128 pixels) that wastes the fewest accumulator rows
     long long best_cost = -1; int btw = 1, bth = 1;
-    const int max_tw = d->stride == 2 ? 128 : 128;
-    for (int tw = 1; tw <= d->out_w && tw <= max_tw; ++tw) {
+    for (int tw = 1; tw <= d->out_w && tw <= 128; ++tw) {
       int th = 128 / tw;
       if (th > d->out_h) th = d->out_h;
       if (th < 1) continue;
@@ -1138,7 +1100,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
     p.epi_groups = num_k_total * (p.KC / 16) * p.BN <= 4096 ? 3 : 2;   // MMA cycles per tile ~ k-steps * BN / 2
     if (p.epi_groups > p.acc_stages) p.epi_groups = p.acc_stages;
     if (d->epilogue == YX_EPI_HEAD && p.epi_groups > 2) p.epi_groups = 2;   // staging slabs are 10.9 KB per warp
-    if (const char* e = getenv("YX_EPI_GROUPS")) { int v = atoi(e); if (v >= 1 && v <= kMaxEpiGroups && v <= p.acc_stages) p.epi_groups = v; }
     if (ctas == 2) p.epi_groups = 1;
   }
   p.head_bytes = d->epilogue == YX_EPI_HEAD ? (((unsigned)p.epi_groups * 4u * 32u * (unsigned)(5 + d->head_nc) * 4u + 1023u) & ~1023u) : 0u;
@@ -1202,7 +1163,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(W) failed: %d", (int)r);
   }
-  p.pdl_late = (getenv("YX_PDL_EARLY") && getenv("YX_PDL_EARLY")[0] == '0') ? 0 : 1;
   p.mul_tpi = fast_div_mul(p.tiles_w * p.tiles_h);
   p.mul_tw = fast_div_mul(p.tiles_w);
   p.mul_ntiles = fast_div_mul(p.n_tiles);
@@ -1270,11 +1230,8 @@ int conv_tc_launch(const ConvTcLaunch* L, cudaStream_t stream) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   const bool silu = L->p.epi.act == YX_ACT_SILU && L->p.epi.epilogue == YX_EPI_STORE;
-#ifdef YX_CONV_TRACE
-  { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(g_conv_trace, z, sizeof(z)); }
-#endif
   const bool head = L->p.epi.epilogue == YX_EPI_HEAD;
   if (L->p.epi.dtype == YX_FP16) {
     if (head) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true>, L->map_a, L->map_b, L->p));
@@ -1285,17 +1242,6 @@ int conv_tc_launch(const ConvTcLaunch* L, cudaStream_t stream) {
     else if (silu) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, false>, L->map_a, L->map_b, L->p));
     else YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false>, L->map_a, L->map_b, L->p));
   }
-#ifdef YX_CONV_TRACE
-  {
-    unsigned long long z[16];
-    cudaStreamSynchronize(stream);
-    if (cudaMemcpyFromSymbol(z, g_conv_trace, sizeof(z)) == cudaSuccess) {
-      fprintf(stderr, "conv trace (ns from CTA 0 entry): setup %lld | producer: pdl %lld first A issued %lld | mma: weights %lld first A %lld first tile committed %lld | epilogue: first acc %lld first tile stored %lld last tile stored %lld | exit %lld\n",
-              (long long)(z[1] - z[0]), (long long)(z[2] - z[0]), (long long)(z[3] - z[0]), (long long)(z[4] - z[0]), (long long)(z[5] - z[0]),
-              (long long)(z[6] - z[0]), (long long)(z[7] - z[0]), (long long)(z[8] - z[0]), (long long)(z[9] - z[0]), (long long)(z[10] - z[0]));
-    }
-  }
-#endif
   return YX_OK;
 }
 

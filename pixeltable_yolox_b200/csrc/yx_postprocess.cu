@@ -41,7 +41,7 @@ static constexpr int kNmsFixedBytes = kChunkBytes + kChunk * 4 + 3 * kClassCap *
 static constexpr int kKeptEntryBytes = 20;  // box 16 + (class | next << 10) 4; the area is recomputed (3 flops)
 static constexpr int kNmsSmemBudget = 224 * 1024;   // dynamic shared memory (+ ~3.5 KB static <= 228 KB per CTA): 8 704 kept entries, i.e. every anchor of a 640^2 image
 
-static constexpr int kFlushRows = 192;               // survivor batch: resolved once it holds this many of its 512 rows (measured sweep 128..512: flat within 3 %, profiles/r2_nms_flush_sweep.jsonl; YX_NMS_FLUSH overrides)
+static constexpr int kFlushRows = 192;               // survivor batch: resolved once it holds this many of its 512 rows (measured sweep 128..512: flat within 3 %, profiles/r2_nms_flush_sweep.jsonl)
 static constexpr int kNmsMaxCluster = 8;             // CTAs of one image's thread-block cluster (sort_nms_kernel<true>)
 
 __device__ __forceinline__ uint32_t orderable(float f) { return orderable_f32(f); }
@@ -214,7 +214,6 @@ struct NmsArgs {
   long long gkeys_stride;          // keys per image in gkeys (next_pow2(per_image))
   int smem_keys_cap;               // number of 64-bit keys the dynamic shared memory can hold
   int smem_bytes;                  // dynamic shared memory of the launch
-  int flush_rows;                  // a batch of phase-A survivors is resolved once it holds this many rows
   int kept_cap;                    // kept boxes that fit the shared-memory kept list
   float4* sorted_box;              // boxes as NMS sees them (offset applied for variant 0)
   int* sorted_cls;
@@ -223,7 +222,6 @@ struct NmsArgs {
   // outputs
   int* keep; int* keep_count;      // yx_batched_nms
   float* dets; long long* det_idx; int* det_count; int max_det;  // yx_postprocess (from cand rows)
-  int debug;                       // YX_NMS_DEBUG: thread 0 prints per-phase cycle counts
   int no_small;                    // YX_NMS_NO_SMALL: never take the single-warp path (tests compare the two paths)
 };
 
@@ -501,15 +499,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
   int* kept = g.kept_pos + base;
 
   if (tid == 0) s_nkept = 0;
-  long long tk[8];
-  long long acc_a = 0, acc_b = 0, acc_c = 0, acc_d = 0, t_prev = 0;   // YX_NMS_DEBUG: clocks per phase over all groups / batches
-#ifdef YX_NMS_TRACE
-  long long tr[6] = {0, 0, 0, 0, 0, 0};
-#define YX_TR(k) { tr[k] += clock64() - t_prev; }
-#else
-#define YX_TR(k)
-#endif
-  tk[0] = clock64();
   // torchvision.ops.batched_nms: coordinate trick unless boxes.numel() > 100000 (CUDA, torchvision >= 0.19; the installed
   // 0.26 the goldens were generated with) / 4000 (CPU) / 20000 (CUDA, torchvision 0.17.2 = the reference's poetry.lock pin)
   int variant = g.variant;
@@ -592,7 +581,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
         cmax = max(cmax, s_xi[rr * 2]); cmin = min(cmin, s_xi[rr * 2 + 1]);
       }
     }
-    tk[1] = clock64();
     // ---------------- gather the sorted candidates (four rows in flight per thread) ----------------
     // boxes_for_nms = boxes + idxs.to(boxes) * (max_coordinate + 1)   (torchvision boxes.py) for the offset variant.
     // With a cluster the position of a key is its index in the own run plus its lower bounds in the other runs
@@ -646,7 +634,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
     }
     if constexpr (CL) nms_cluster_sync(); else __syncthreads();   // sorted rows visible; runs no longer read
 
-    tk[2] = clock64();
     // ---------------- greedy NMS: groups of 512 candidates, batches of survivors ----------------
     // Which pairs can interact?  per-class variant: equal classes only.  Offset variant: class c lives in
     // [c*s + min, c*s + max] with s = max+1, so classes a < b can only overlap when (b-a)*s < max-min+1,
@@ -702,7 +689,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
     int g0 = 0;                       // first candidate of the group
     int nb = 0, cbase = 0;            // rows in the batch; sorted position of its first group (s_cpos is relative to it)
     unsigned turn = 0;                // phase-A executions so far: parity selects the dead-bit exchange buffer
-    t_prev = clock64();
     while (g0 < n || nb > 0) {
       __syncthreads();
       const int nk = s_nkept;
@@ -714,7 +700,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
         const int my_cls = cur_cls;
         const float my_area = box_area(me);
         bool dead = (tid >= gn);
-        YX_TR(0)
         // ---- phase A: against the boxes kept so far
         if (!dead) {
           const int nks = min(nk_own, KC);
@@ -750,7 +735,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
             if (suppresses(kb, box_area(kb), me, my_area, g.thr)) dead = true;
           }
         }
-        YX_TR(1)
         {
           const unsigned bal = __ballot_sync(0xffffffffu, dead);
           if constexpr (CL) {
@@ -778,7 +762,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
           before += l < warp ? pc : 0;
         }
         const bool alive = !((s_removed[warp] >> lane) & 1u);
-        { const long long t = clock64(); acc_a += t - t_prev; t_prev = t; }
         if (nb + surv <= kChunk) {
           if (nb == 0) cbase = g0;
           if (alive) {
@@ -791,7 +774,7 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
           cur_box = nx_box; cur_cls = nx_cls;
           if (g0 + kChunk + tid < n) { nx_box = sbox[g0 + kChunk + tid]; nx_cls = scls[g0 + kChunk + tid]; }
           // resolve the batch when it is nearly full, at the end of the list, or before its 16-bit positions run out
-          flush = nb >= g.flush_rows || g0 >= n || g0 - cbase > 60000;
+          flush = nb >= kFlushRows || g0 >= n || g0 - cbase > 60000;
         }
         // else: the batch is resolved first and the group tested again
       }
@@ -805,7 +788,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
         // items (row, word): 16 per row, the words before the row's own are skipped; with a cluster the items are
         // dealt round-robin over the CTAs and stored into CTA 0's mask
         const int items = cn << 4;
-        YX_TR(2)
         for (int q = rank * kNmsThreads + tid; q < items; q += R * kNmsThreads) {
           const int row = q >> 4;
           const int w = q & (kChunkWords - 1);
@@ -838,10 +820,8 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
           }
           cmask_w[row * kMaskPitch + w] = bits;
         }
-        YX_TR(3)
         if constexpr (CL) nms_cluster_sync(); else __syncthreads();   // (2) CTA 0 holds the whole mask
       }
-      { const long long t = clock64(); acc_b += t - t_prev; t_prev = t; }
       // ---- phase C: one warp walks the batch word by word (32 rows); lane l owns word l of the removed set (at the
       //      start: the rows past the end of the batch). Inside a word the greedy order is resolved on the 32x32 diagonal
       //      block held in registers; the rows of the kept boxes are then OR-ed into the later words.
@@ -903,10 +883,8 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
           }
         }
         if (lane == 0) s_ck = cnt;
-        YX_TR(4)
       }
       if constexpr (CL) nms_cluster_sync(); else __syncthreads();     // (3) CTA 0 has the batch's survivors
-      { const long long t = clock64(); acc_c += t - t_prev; t_prev = t; }
       // ---- append the batch's survivors to the kept list (parallel; list order is irrelevant)
       {
         // (the other CTAs read CTA 0's list: it is rewritten only after barrier (2) of the next batch)
@@ -933,7 +911,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
       }
       nb = 0;
       __syncthreads();
-      { const long long t = clock64(); acc_d += t - t_prev; t_prev = t; }
     }
     if constexpr (CL) nms_cluster_sync();   // the other CTAs have read the last batch's survivors from CTA 0
   }
@@ -942,7 +919,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
 
   // ---------------- outputs ----------------
   const int nk = s_nkept;
-  tk[6] = clock64();
   if (g.keep) {
     for (int k = tid; k < nk; k += kNmsThreads) g.keep[base + k] = sidx[kept[k]];
     if (tid == 0) g.keep_count[b] = nk;
@@ -959,14 +935,6 @@ __global__ void __launch_bounds__(kNmsThreads, 1) sort_nms_kernel(const NmsArgs 
     }
     if (tid == 0) g.det_count[b] = nk;  // true number kept; rows beyond max_det are dropped
   }
-  if (g.debug && tid == 0 && n > 0)
-    printf("nms b=%d R=%d n=%d kept=%d keys+sort=%lld gather=%lld A=%lld B=%lld C=%lld append=%lld out=%lld\n", b, R, n, nk,
-           tk[1] - tk[0], tk[2] - tk[1], acc_a, acc_b, acc_c, acc_d, clock64() - tk[6]);
-#ifdef YX_NMS_TRACE
-  if (g.debug && tid == 0 && n > 0)
-    printf("trace b=%d (since phase start) A: loaded=%lld walked=%lld | B: compacted=%lld items=%lld | C: scanned=%lld\n", b,
-           tr[0], tr[1], tr[2], tr[3], tr[4]);
-#endif
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1063,10 +1031,7 @@ static int launch_sort_nms(NmsArgs& g, int batch, cudaStream_t s) {
   g.smem_keys_cap = smem_keys_cap(g.src.per_image);
   g.kept_cap = kept_cap_for(g.src.per_image);
   g.gkeys_stride = next_pow2_ll(g.src.per_image);
-  g.debug = getenv("YX_NMS_DEBUG") ? 1 : 0;
   g.no_small = getenv("YX_NMS_NO_SMALL") ? 1 : 0;
-  g.flush_rows = kFlushRows;
-  if (const char* e = getenv("YX_NMS_FLUSH")) { const int v = atoi(e); if (v >= 32 && v <= kChunk) g.flush_rows = v; }
   const size_t smem = nms_smem_bytes(g.src.per_image);
   g.smem_bytes = (int)smem;
   static size_t configured_dev[kMaxDevices] = {};

@@ -30,13 +30,13 @@ static constexpr int kStemBuilders = 128;            // threads per builder grou
 static constexpr int kStemMaxRing = 4;               // barrier arrays are sized for the largest variant
 // Variant V: 0 = one CTA per SM (two builder groups, two issuing warps, four epilogue groups, 4-deep rings);
 //            1 = two co-resident CTAs per SM with half of everything each (one builder group, one issuing warp, two
-//                epilogue groups, 2-deep rings); 2 = like 1 with ONE epilogue group (320 threads: no register squeeze).
+//                epilogue groups, 2-deep rings).
 // The single-CTA kernel is bound by the hand-off latency of its TMA -> builder -> MMA -> epilogue pipeline (~1 000 clk per
 // 120-pixel tile with no unit saturated, section 4.4 of DESIGN.md); two independent pipelines per SM overlap that latency.
 template <int V> struct StemCfg {
   static constexpr int kBuilderGroups = V == 0 ? 2 : 1;       // tiles alternate between the groups
   static constexpr int kMmaWarps = V == 0 ? 2 : 1;            // tiles alternate between the issuing warps
-  static constexpr int kEpiGroups = V == 0 ? 4 : (V == 1 ? 2 : 1);
+  static constexpr int kEpiGroups = V == 0 ? 4 : 2;
   static constexpr int kStages = V == 0 ? 4 : 2;              // halo-tile (A operand) stages
   static constexpr int kAcc = V == 0 ? 4 : 2;
   static constexpr int kPatchStages = V == 0 ? 4 : 2;
@@ -69,13 +69,8 @@ struct StemParams {
   int BN, BNpad;              // out_c (multiple of 16) and its TMEM pitch
   unsigned idesc, desc_hi, tmem_cols;
   unsigned bias_bytes, b_bytes, w_tile_bytes, patch_tx;
-  int debug;
   EpiParams epi;
 };
-
-// YX_STEM_DEBUG=2: CTA 0 records clock64() at the hand-off points of tiles 16..47 (builder warp 0, MMA warp, epilogue warp 0)
-__device__ long long g_stem_trace[3][32][5];
-#define ST_TRACE(role, it, k) do { if ((p.debug & 2) && blockIdx.x == 0 && (it) >= 16 && (it) < 48 && lane == 0) g_stem_trace[role][(it) - 16][k] = clock64(); } while (0)
 
 struct __align__(8) StemShared {
   uint64_t full[kStemMaxRing];
@@ -187,12 +182,9 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
       if (tl >= p.num_tiles) break;
       const int stage = it % kStemStages, ps = it % kPatchStages;
       const uint32_t phase = (uint32_t)((it / kStemStages) & 1), pphase = (uint32_t)((it / kPatchStages) & 1);
-      if (warp == 0) ST_TRACE(0, it, 0);
       mbar_wait(&sh->patch_full[ps], pphase);
-      if (warp == 0) ST_TRACE(0, it, 1);
       const TI* pt = reinterpret_cast<const TI*>(patch + (size_t)ps * p.patch_stage_bytes);
       mbar_wait(&sh->empty[stage], phase ^ 1);
-      if (warp == 0) ST_TRACE(0, it, 2);
       uint8_t* a0 = astage + (size_t)stage * p.a_stage_bytes;
       float fa[2][6], fb[2][6];
 #pragma unroll
@@ -218,21 +210,19 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
           *reinterpret_cast<uint4*>(a0 + row1[rep]) = make_uint4(wd[4], wd[5], 0u, 0u);
         }
       }
-      if (warp == 0) ST_TRACE(0, it, 3);
       fence_proxy_async();                    // this thread's generic-proxy stores -> visible to the tensor core
       __syncwarp();
       if (lane == 0) {
         mbar_arrive(&sh->patch_empty[ps]);    // the warp is done with the raw patch
         mbar_arrive(&sh->full[stage]);
       }
-      if (warp == 0) ST_TRACE(0, it, 4);
     }
   } else if (warp == kWarpMma || (kMmaWarps == 2 && warp == kWarpMma2)) {
     // ===================== MMA issuers =====================
     // A [128 x 16] x [16 x 32] MMA is bound by the tensor core's shared-memory read of A (128 rows x 32 B at ~64 B/clk =
     // 64 clk, the math needs 16) and the issuing thread stays in tcgen05.mma for about that long, so its barrier waits
     // (~150 clk each even when the phase is already complete) were dead time of the tensor pipe: a clock64 trace
-    // (YX_STEM_DEBUG=2) showed 780 clk of issue + 420 clk of waits per tile. Two warps issue alternate tiles.
+    // showed 780 clk of issue + 420 clk of waits per tile. Two warps issue alternate tiles.
     const int g = warp == kWarpMma ? 0 : 1;
     if (lane == 0) {
       if (g == 0) {
@@ -249,11 +239,8 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         if (tl >= p.num_tiles) break;
         const int stage = mit % kStemStages, as = mit % kStemAcc;
         const uint32_t phase = (uint32_t)((mit / kStemStages) & 1), aphase = (uint32_t)((mit / kStemAcc) & 1);
-        ST_TRACE(1, mit, 0);
         mbar_wait(&sh->tmem_empty[as], aphase ^ 1);
-        ST_TRACE(1, mit, 1);
         mbar_wait(&sh->full[stage], phase);
-        ST_TRACE(1, mit, 2);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BNpad);
         const uint32_t a16 = smem_u32(astage + (size_t)stage * p.a_stage_bytes) >> 4;
@@ -266,7 +253,6 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         }
         umma_commit(&sh->empty[stage]);
         umma_commit(&sh->tmem_full[as]);
-        ST_TRACE(1, mit, 3);
       }
     }
   } else if (warp == kWarpTma) {
@@ -280,13 +266,9 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         const int r = t - b * tiles_per_img;
         const int ty = r / p.tiles_w, tx = r - ty * p.tiles_w;
         mbar_wait(&sh->patch_empty[ps], pphase ^ 1);
-        if (p.debug & 1) {
-          mbar_arrive(&sh->patch_full[ps]);
-        } else {
-          mbar_arrive_expect_tx(&sh->patch_full[ps], p.patch_tx);
-          tma_load_4d(&map_img, &sh->patch_full[ps], patch + (size_t)ps * p.patch_stage_bytes,
-                      2 * tx * p.tw - 2 - p.lead, 2 * ty * p.th - 2, 0, b);
-        }
+        mbar_arrive_expect_tx(&sh->patch_full[ps], p.patch_tx);
+        tma_load_4d(&map_img, &sh->patch_full[ps], patch + (size_t)ps * p.patch_stage_bytes,
+                    2 * tx * p.tw - 2 - p.lead, 2 * ty * p.th - 2, 0, b);
         if (++ps == kPatchStages) { ps = 0; pphase ^= 1; }
       }
     }
@@ -309,9 +291,7 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
       const int ty = fast_div(r, p.mul_tw, p.tiles_w), tx = r - ty * p.tiles_w;
       const int ho = ty * p.th + hl, wo = tx * p.tw + wl;
       const bool valid = row_ok && ho < p.out_h && wo < p.out_w;
-      if (warp == kWarpEpi) ST_TRACE(2, it, 0);
       mbar_wait(&sh->tmem_full[as], aphase);
-      if (warp == kWarpEpi) ST_TRACE(2, it, 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(as * p.BNpad);
       const long long pix = ((long long)b * p.out_h + ho) * p.out_w + wo;
@@ -322,17 +302,14 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
         tmem_ld_x16(taddr + (uint32_t)c, ra);
         if (two) tmem_ld_x16(taddr + (uint32_t)(c + 16), rb);
         tmem_ld_wait();
-        if (warp == kWarpEpi && c == 0) ST_TRACE(2, it, 2);
         if (valid) {
           epi_tc_chunk<FP16, SILU>(p.epi, ra, sbias + c, nullptr, orow + c, b, ho, wo, c);
           if (two) epi_tc_chunk<FP16, SILU>(p.epi, rb, sbias + c + 16, nullptr, orow + c + 16, b, ho, wo, c + 16);
         }
       }
-      if (warp == kWarpEpi) ST_TRACE(2, it, 3);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&sh->tmem_empty[as]);
-      if (warp == kWarpEpi) ST_TRACE(2, it, 4);
     }
   }
 
@@ -361,15 +338,10 @@ struct StemLaunch {
   int variant;            // StemCfg<V>
 };
 
-// ring depths / thread counts of the variants for the host side (same numbers as StemCfg<V>)
-// Default: two co-resident CTAs (variant 1) when they fit. Measured at 64 x 640^2 (tools/gpu_time_stem.py): 210 -> 202 us
-// (fp32 image), 214 -> 201 us (uint8); variant 2 (one epilogue group per CTA) 216 us. The gain is small because the kernel
-// is not latency-bound after all: ncu (profiles/r2_stem.md) has the L1 data pipe saturated -- LSU wavefronts 68 % (shared
-// loads of the builders and epilogues 39 %, stores 9 %) + tensor-core operand reads 34 % of the same pipe.
-static int stem_variant() {
-  if (const char* e = getenv("YX_STEM_V")) { const int v = atoi(e); if (v >= 0 && v <= 2) return v; }
-  return 1;
-}
+// Two co-resident CTAs (variant 1) when they fit. Measured at 64 x 640^2 (tools/gpu_time_stem.py): 210 -> 202 us
+// (fp32 image), 214 -> 201 us (uint8); a variant with one epilogue group per CTA measured 216 us. The gain is small because
+// the kernel is not latency-bound after all: ncu (profiles/r2_stem.md) has the L1 data pipe saturated -- LSU wavefronts 68 %
+// (shared loads of the builders and epilogues 39 %, stores 9 %) + tensor-core operand reads 34 % of the same pipe.
 
 StemLaunch* stem_alloc() {
   void* p = nullptr;
@@ -407,10 +379,6 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
       const long long cost = tiles * 3 * (2 * th + 4);
       if (best < 0 || cost < best) { best = cost; p.tw = tw; p.th = th; }
     }
-    if (const char* e = getenv("YX_STEM_TILE")) {          // experiments: "tw"
-      const int tw = atoi(e);
-      if (tw >= 8 && tw <= 126 && (2 * tw * es0) % 16 == 0) { p.tw = tw; p.th = 128 / (tw + 2); }
-    }
   }
   p.pitch = p.tw + 2; p.halo_pix = (p.th + 2) * p.pitch;
   YX_REQUIRE(p.halo_pix <= 2 * kStemBuilders, YX_ERR_UNSUPPORTED, "stem: halo of %d pixels exceeds the builder groups", p.halo_pix);
@@ -420,7 +388,7 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
   p.mul_tpi = fast_div_mul(p.tiles_w * p.tiles_h); p.mul_tw = fast_div_mul(p.tiles_w);
   p.BN = out_c;
   p.BNpad = 32; while (p.BNpad < p.BN) p.BNpad <<= 1;
-  int V = stem_variant();
+  int V = 1;
   {
     // two CTAs per SM need <= 112 KB each; otherwise fall back to the single-CTA variant
     const unsigned es1 = img_dtype == YX_FP32 ? 4u : 1u;
@@ -429,7 +397,7 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
     const size_t patch1 = ((size_t)(3 * p.patch_rows) * pitch1 * es1 + 127u) & ~(size_t)127u;
     const size_t a1 = ((size_t)(128 + 2 * p.pitch + 2) * 32u + 1023u) & ~(size_t)1023u;
     const size_t need = 2048 + ((size_t)out_c * 4u + 1023u) / 1024u * 1024u + 2 * patch1 + 1024 + (((size_t)out_c * 32u * 9u + 1023u) & ~(size_t)1023u) + 2 * a1;
-    if (V != 0 && need > 112 * 1024) V = 0;
+    if (need > 112 * 1024) V = 0;
   }
   L->variant = V;
   const int n_acc = V == 0 ? StemCfg<0>::kAcc : StemCfg<1>::kAcc;
@@ -471,7 +439,6 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     YX_REQUIRE(ri == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(stem image) failed: %d", (int)ri);
     p.patch_tx = bw * (cuuint32_t)p.patch_rows * 3 * es;
-    if (const char* e = getenv("YX_STEM_DEBUG")) p.debug = atoi(e);
   }
   const CUtensorMapDataType tdt = dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   cuuint64_t dims[2] = {144, (cuuint64_t)out_c};
@@ -493,7 +460,7 @@ int stem_launch(const StemLaunch* L, cudaStream_t stream) {
 #define YX_STEM_ATTR1(T, F, V) \
   YX_CUDA(cudaFuncSetAttribute(stem_tc_kernel<T, F, true, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, V == 0 ? 200 * 1024 : 112 * 1024)); \
   YX_CUDA(cudaFuncSetAttribute(stem_tc_kernel<T, F, false, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, V == 0 ? 200 * 1024 : 112 * 1024))
-#define YX_STEM_ATTR(T, F) YX_STEM_ATTR1(T, F, 0); YX_STEM_ATTR1(T, F, 1); YX_STEM_ATTR1(T, F, 2)
+#define YX_STEM_ATTR(T, F) YX_STEM_ATTR1(T, F, 0); YX_STEM_ATTR1(T, F, 1)
     YX_STEM_ATTR(float, false); YX_STEM_ATTR(float, true); YX_STEM_ATTR(uint8_t, false); YX_STEM_ATTR(uint8_t, true);
 #undef YX_STEM_ATTR
 #undef YX_STEM_ATTR1
@@ -503,19 +470,19 @@ int stem_launch(const StemLaunch* L, cudaStream_t stream) {
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)L->grid);
   const int V = L->variant;
-  cfg.blockDim = dim3((unsigned)(V == 0 ? StemCfg<0>::kThreads : (V == 1 ? StemCfg<1>::kThreads : StemCfg<2>::kThreads)));
+  cfg.blockDim = dim3((unsigned)(V == 0 ? StemCfg<0>::kThreads : StemCfg<1>::kThreads));
   cfg.dynamicSmemBytes = L->smem;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   const bool h16 = L->p.epi.dtype == YX_FP16;
   const bool silu = L->p.epi.act == YX_ACT_SILU;
 #define YX_STEM_GO1(T, F, V) do { if (silu) YX_CUDA(cudaLaunchKernelEx(&cfg, stem_tc_kernel<T, F, true, V>, L->map_w, L->map_img, L->p)); \
     else YX_CUDA(cudaLaunchKernelEx(&cfg, stem_tc_kernel<T, F, false, V>, L->map_w, L->map_img, L->p)); } while (0)
-#define YX_STEM_GO(T, F) do { if (V == 0) YX_STEM_GO1(T, F, 0); else if (V == 1) YX_STEM_GO1(T, F, 1); else YX_STEM_GO1(T, F, 2); } while (0)
+#define YX_STEM_GO(T, F) do { if (V == 0) YX_STEM_GO1(T, F, 0); else YX_STEM_GO1(T, F, 1); } while (0)
   if (L->p.img_dtype == YX_FP32) {
     if (h16) YX_STEM_GO(float, true); else YX_STEM_GO(float, false);
   } else {
@@ -523,21 +490,6 @@ int stem_launch(const StemLaunch* L, cudaStream_t stream) {
   }
 #undef YX_STEM_GO
 #undef YX_STEM_GO1
-  if (L->p.debug & 2) {
-    static long long tr[3][32][5];
-    cudaStreamSynchronize(stream);
-    if (cudaMemcpyFromSymbol(tr, g_stem_trace, sizeof(tr)) == cudaSuccess) {
-      const char* names[3] = {"builder", "mma", "epilogue"};
-      const long long t0 = tr[1][0][0];
-      for (int r = 0; r < 3; ++r)
-        for (int i = 0; i < 32; ++i) {
-          if (tr[r][i][0] == 0) continue;
-          fprintf(stderr, "stem trace %-8s it=%2d:", names[r], i + 16);
-          for (int k = 0; k < 5; ++k) fprintf(stderr, " %7lld", tr[r][i][k] ? tr[r][i][k] - t0 : -1);
-          fprintf(stderr, "\n");
-        }
-    }
-  }
   return YX_OK;
 }
 

@@ -302,11 +302,10 @@ __device__ __forceinline__ float tanh_approx(float x) {
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(x));
   return t;
 }
-// act bit 8 (YX_BN_PRECISE=1 in the environment): keep the ex2 + division form for bf16 too (A/B of the approximation)
 template <bool FAST>
 __device__ __forceinline__ float bn_act_t(float z, int act) {
   if (FAST && act == YX_ACT_SILU) { const float h = 0.5f * z; return fmaf(h, tanh_approx(h), h); }
-  return bn_act(z, act & 0xff);
+  return bn_act(z, act);
 }
 __device__ __forceinline__ float bn_act_grad(float z, int act);
 template <bool FAST>
@@ -315,7 +314,7 @@ __device__ __forceinline__ float bn_act_grad_t(float z, int act) {
     const float s = fmaf(0.5f, tanh_approx(0.5f * z), 0.5f);
     return s * fmaf(z, 1.0f - s, 1.0f);
   }
-  return bn_act_grad(z, act & 0xff);
+  return bn_act_grad(z, act);
 }
 __device__ __forceinline__ float bn_act_grad(float z, int act) {
   if (act == YX_ACT_SILU) { const float s = 1.0f / (1.0f + __expf(-z)); return s * (1.0f + z * (1.0f - s)); }
@@ -586,12 +585,6 @@ long long bn_act_ws_bytes(int n, int c, int hw) {
   return (((long long)c * parts * 2 * 4) + 255) & ~255LL;
 }
 
-static int bn_precise_flag() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("YX_BN_PRECISE"); v = (e && e[0] == '1') ? 0x100 : 0; }
-  return v;
-}
-
 static int bn_check(int dtype, int n, int c, int hw, int act) {
   YX_REQUIRE(dtype == YX_FP32 || dtype == YX_BF16 || dtype == YX_FP16, YX_ERR_INVALID_ARG, "bn_act: dtype %d", dtype);
   YX_REQUIRE(n > 0 && c > 0 && hw > 0 && n <= 65535 && c <= 65535, YX_ERR_INVALID_ARG, "bn_act: bad sizes");
@@ -614,11 +607,11 @@ int bn_act_train_fwd_launch(const void* x, int dtype, int nhwc, int n, int c, in
     const long long M = (long long)n * hw;
     int rows = 0, rows2 = 0;
     const int S = bn_nhwc_slabs(M, 64, 4, &rows), S2 = bn_nhwc_slabs(M, 32, 6, &rows2);
-#define YX_GO(T) launch_pdl(bn_reduce_nhwc_kernel<T, false, 4>, dim3(S), dim3(kBnThreads), 0, s, (const T*)x, nullptr, nullptr, nullptr, nullptr, nullptr, M, c, rows, act | bn_precise_flag(), part, (long long)c)
+#define YX_GO(T) launch_kernel(bn_reduce_nhwc_kernel<T, false, 4>, dim3(S), dim3(kBnThreads), 0, s, (const T*)x, nullptr, nullptr, nullptr, nullptr, nullptr, M, c, rows, act, part, (long long)c)
     if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
-    launch_pdl(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, S, (double)M, eps, momentum, running_mean, running_var, save_mean, save_invstd, 0, nbt, (float*)nullptr, (float*)nullptr);
-#define YX_GO(T) launch_pdl(bn_apply_nhwc_kernel<T, false, 4>, dim3(S2), dim3(kBnThreads), 0, s, (const T*)x, nullptr, save_mean, save_invstd, gamma, beta, nullptr, nullptr, 0.0f, M, c, rows2, act | bn_precise_flag(), (T*)y, (long long)c)
+    launch_kernel(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, S, (double)M, eps, momentum, running_mean, running_var, save_mean, save_invstd, 0, nbt, (float*)nullptr, (float*)nullptr);
+#define YX_GO(T) launch_kernel(bn_apply_nhwc_kernel<T, false, 4>, dim3(S2), dim3(kBnThreads), 0, s, (const T*)x, nullptr, save_mean, save_invstd, gamma, beta, nullptr, nullptr, 0.0f, M, c, rows2, act, (T*)y, (long long)c)
     if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
     YX_CUDA(cudaGetLastError());
@@ -626,12 +619,12 @@ int bn_act_train_fwd_launch(const void* x, int dtype, int nhwc, int n, int c, in
   }
   const int chunks = (hw + kBnChunk - 1) / kBnChunk;
   const dim3 grid((unsigned)chunks, (unsigned)c, (unsigned)n);
-#define YX_GO(T) launch_pdl(bn_reduce_kernel<T, false>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, nullptr, nullptr, nullptr, nullptr, nullptr, c, hw, act, part)
+#define YX_GO(T) launch_kernel(bn_reduce_kernel<T, false>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, nullptr, nullptr, nullptr, nullptr, nullptr, c, hw, act, part)
   if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
-  launch_pdl(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, n * chunks, (double)n * hw, eps, momentum, running_mean, running_var,
+  launch_kernel(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, n * chunks, (double)n * hw, eps, momentum, running_mean, running_var,
                                                      save_mean, save_invstd, 0, nbt, (float*)nullptr, (float*)nullptr);
-#define YX_GO(T) launch_pdl(bn_apply_kernel<T, false>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, nullptr, save_mean, save_invstd, gamma, beta, nullptr, nullptr, 0.0f, c, hw, act, (T*)y)
+#define YX_GO(T) launch_kernel(bn_apply_kernel<T, false>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, nullptr, save_mean, save_invstd, gamma, beta, nullptr, nullptr, 0.0f, c, hw, act, (T*)y)
   if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
   YX_CUDA(cudaGetLastError());
@@ -655,12 +648,12 @@ int bn_act_train_bwd_launch(const void* x, const void* dy, int dtype, int nhwc, 
     const long long M = (long long)n * hw;
     int rows = 0, rows2 = 0;
     const int S = bn_nhwc_slabs(M, 64, 4, &rows), S2 = bn_nhwc_slabs(M, 32, 6, &rows2);
-#define YX_GO(T) launch_pdl(bn_reduce_nhwc_kernel<T, true, 2>, dim3(S), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, M, c, rows, act | bn_precise_flag(), part, dy_ld)
+#define YX_GO(T) launch_kernel(bn_reduce_nhwc_kernel<T, true, 2>, dim3(S), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, M, c, rows, act, part, dy_ld)
     if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
-    launch_pdl(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, S, (double)M, 0.0f, 0.0f, nullptr, nullptr, dbeta, dgamma, 1, (long long*)nullptr, acc_dbeta, acc_dgamma);
+    launch_kernel(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, S, (double)M, 0.0f, 0.0f, nullptr, nullptr, dbeta, dgamma, 1, (long long*)nullptr, acc_dbeta, acc_dgamma);
     const float inv_m = (float)(1.0 / (double)M);
-#define YX_GO(T) launch_pdl(bn_apply_nhwc_kernel<T, true, 2>, dim3(S2), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, dbeta, dgamma, inv_m, M, c, rows2, act | bn_precise_flag(), (T*)dx, dy_ld)
+#define YX_GO(T) launch_kernel(bn_apply_nhwc_kernel<T, true, 2>, dim3(S2), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, dbeta, dgamma, inv_m, M, c, rows2, act, (T*)dx, dy_ld)
     if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
     YX_CUDA(cudaGetLastError());
@@ -668,12 +661,12 @@ int bn_act_train_bwd_launch(const void* x, const void* dy, int dtype, int nhwc, 
   }
   const int chunks = (hw + kBnChunk - 1) / kBnChunk;
   const dim3 grid((unsigned)chunks, (unsigned)c, (unsigned)n);
-#define YX_GO(T) launch_pdl(bn_reduce_kernel<T, true>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, c, hw, act, part)
+#define YX_GO(T) launch_kernel(bn_reduce_kernel<T, true>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, c, hw, act, part)
   if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
-  launch_pdl(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, n * chunks, (double)n * hw, 0.0f, 0.0f, nullptr, nullptr, dbeta, dgamma, 1, (long long*)nullptr, acc_dbeta, acc_dgamma);
+  launch_kernel(bn_finalize_kernel, dim3((c + 3) / 4), dim3(128), 0, s, part, c, n * chunks, (double)n * hw, 0.0f, 0.0f, nullptr, nullptr, dbeta, dgamma, 1, (long long*)nullptr, acc_dbeta, acc_dgamma);
   const float inv_m = (float)(1.0 / ((double)n * hw));
-#define YX_GO(T) launch_pdl(bn_apply_kernel<T, true>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, dbeta, dgamma, inv_m, c, hw, act, (T*)dx)
+#define YX_GO(T) launch_kernel(bn_apply_kernel<T, true>, dim3(grid), dim3(kBnThreads), 0, s, (const T*)x, (const T*)dy, save_mean, save_invstd, gamma, beta, dbeta, dgamma, inv_m, c, hw, act, (T*)dx)
   if (dtype == YX_FP32) YX_GO(float); else if (dtype == YX_BF16) YX_GO(__nv_bfloat16); else YX_GO(__half);
 #undef YX_GO
   YX_CUDA(cudaGetLastError());

@@ -334,17 +334,15 @@ static int wgrad_plan(int batch, int in_h, int in_w, int in_c, int out_h, int ou
   p.n_blocks = p.N / p.ci_box;
   p.Ncol = (p.N + 31) & ~31;
   p.slices = p.n_tiles * p.taps;
-  // slices per CTA: measured on the yolox_s layers (tools/gpu_wgrad_sweep.py), about 128 accumulator columns per CTA is best
+  // slices per CTA: measured on the yolox_s layers by sweeping it, about 128 accumulator columns per CTA is best
   // (N = 128: one slice, 36.6 -> 20.8 us for 256->256 3x3 @20x20; N = 64: two; N = 32: four): more CTAs on the (o, i, tap)
   // space and a shorter epilogue per CTA beat the saved re-loads of the dy tile; N = 16 keeps all nine taps together
   int sg_max = p.N <= 16 ? 512 / p.Ncol : (128 / p.N > 1 ? 128 / p.N : 1);
   if (sg_max > p.slices) sg_max = p.slices;
-  if (const char* e = getenv("YX_WGRAD_SG")) { const int v = atoi(e); if (v >= 1 && v * p.Ncol <= 512) sg_max = v < p.slices ? v : p.slices; }
   p.n_groups = (p.slices + sg_max - 1) / sg_max;
   p.SG = (p.slices + p.n_groups - 1) / p.n_groups;
   p.n_groups = (p.slices + p.SG - 1) / p.SG;
   p.merged = (p.n_blocks == 1 && p.SG > 1 && p.SG * p.N <= 256) ? 1 : 0;
-  if (const char* e = getenv("YX_WGRAD_MERGE")) { if (e[0] == '0') p.merged = 0; }
 
   int dev = 0, max_smem = 0;
   YX_CUDA(cudaGetDevice(&dev));
@@ -353,7 +351,6 @@ static int wgrad_plan(int batch, int in_h, int in_w, int in_c, int out_h, int ou
   const unsigned bpp = 256u + (unsigned)(p.SG * p.N) * 2u;   // bytes per pixel of one stage: 128 A channels + SG * N B channels
   int kp_max = (budget / 3) / (int)bpp / 16 * 16;
   if (kp_max > 128) kp_max = 128;
-  if (const char* e = getenv("YX_WGRAD_KP")) { const int v = atoi(e); if (v >= 16 && v < kp_max) kp_max = v / 16 * 16; }
   if (kp_max < 16) kp_max = 16;
   long long best = -1;
   for (int tw = 1; tw <= 128; ++tw) {
@@ -385,7 +382,6 @@ static int wgrad_plan(int batch, int in_h, int in_w, int in_c, int out_h, int ou
   if (ks < 1) ks = 1;
   if (ks > p.PT) ks = p.PT;
   if (p.PT >= 8 && ks > p.PT / 4) ks = p.PT / 4;          // at least four pixel tiles per CTA: the pipeline needs something to overlap
-  if (const char* e = getenv("YX_WGRAD_KSPLIT")) { const int v = atoi(e); if (v >= 1) ks = v < p.PT ? v : p.PT; }
   p.tiles_per_split = (p.PT + ks - 1) / ks;
   p.ksplit = (p.PT + p.tiles_per_split - 1) / p.tiles_per_split;
   p.row_stride = (long long)p.slices * p.N;
@@ -464,11 +460,11 @@ int wgrad_launch(const void* x, long long x_ld, const void* dy, long long dy_ld,
     attr_set = true;
   }
   const int grid = p.m_tiles * p.n_groups * p.ksplit;
-  cudaError_t e = launch_pdl(wgrad_tc_kernel, dim3(grid), dim3(192), L->smem, stream, L->map_dy, L->map_x, p);
+  cudaError_t e = launch_kernel(wgrad_tc_kernel, dim3(grid), dim3(192), L->smem, stream, L->map_dy, L->map_x, p);
   if (e == cudaSuccess) {
     const long long total = (long long)out_c * p.taps * in_c;
     const int rgrid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-    e = launch_pdl(wgrad_reduce_kernel, dim3(rgrid), dim3(256), 0, stream, (const float*)p.partial, p.ksplit, p.split_stride, p.row_stride,
+    e = launch_kernel(wgrad_reduce_kernel, dim3(rgrid), dim3(256), 0, stream, (const float*)p.partial, p.ksplit, p.split_stride, p.row_stride,
                    p.N, p.taps, out_c, in_c, out_c_real, in_c_real, dw, dw_so, dw_si, dw_st, accumulate);
   }
   free(L);
@@ -485,10 +481,10 @@ int pack_train_weights_launch(const float* w, long long so, long long si, long l
   const long long total = (long long)o_pad * taps * i_pad;
   const int grid = (int)((total + 255) / 256 < 2048 ? (total + 255) / 256 : 2048);
   if (dtype == YX_BF16)
-    YX_CUDA(launch_pdl(pack_train_weights_kernel<__nv_bfloat16>, dim3(grid), dim3(256), 0, stream, w, so, si, st, o, i, taps, o_pad, i_pad,
+    YX_CUDA(launch_kernel(pack_train_weights_kernel<__nv_bfloat16>, dim3(grid), dim3(256), 0, stream, w, so, si, st, o, i, taps, o_pad, i_pad,
                        reinterpret_cast<__nv_bfloat16*>(wf), reinterpret_cast<__nv_bfloat16*>(wd), subpixel));
   else
-    YX_CUDA(launch_pdl(pack_train_weights_kernel<__half>, dim3(grid), dim3(256), 0, stream, w, so, si, st, o, i, taps, o_pad, i_pad,
+    YX_CUDA(launch_kernel(pack_train_weights_kernel<__half>, dim3(grid), dim3(256), 0, stream, w, so, si, st, o, i, taps, o_pad, i_pad,
                        reinterpret_cast<__half*>(wf), reinterpret_cast<__half*>(wd), subpixel));
   return YX_OK;
 }
@@ -506,7 +502,7 @@ int dilate2_launch(const void* dy, void* z, int batch, int oh, int ow, int zh, i
   YX_REQUIRE(dy && z && c % 8 == 0 && batch > 0 && oh > 0 && ow > 0 && zh >= 2 * oh - 1 && zw >= 2 * ow - 1, YX_ERR_INVALID_ARG, "dilate2: shape");
   const long long total = (long long)batch * zh * zw * (c / 8);
   const int grid = (int)((total + 255) / 256 < 8192 ? (total + 255) / 256 : 8192);
-  YX_CUDA(launch_pdl(dilate2_kernel, dim3(grid), dim3(256), 0, stream, reinterpret_cast<const uint4*>(dy), reinterpret_cast<uint4*>(z), batch, oh, ow,
+  YX_CUDA(launch_kernel(dilate2_kernel, dim3(grid), dim3(256), 0, stream, reinterpret_cast<const uint4*>(dy), reinterpret_cast<uint4*>(z), batch, oh, ow,
                      zh, zw, c / 8));
   return YX_OK;
 }

@@ -16,7 +16,6 @@ Data layout in HBM
 from __future__ import annotations
 
 import ctypes as C
-import os
 from dataclasses import dataclass, field
 from typing import Dict, List, Optional, Sequence, Tuple
 
@@ -260,11 +259,9 @@ class Builder:
 
     def bottleneck_fusable(self, x: Feat, m) -> bool:
         """True when Bottleneck `m` can run as the single fused kernel (yx_bottleneck_fwd)."""
-        import os
-
         from .network_blocks import BaseConv
 
-        if os.environ.get("YX_FUSE_BNECK", "1") == "0" or self.dtype == torch.float32:
+        if self.dtype == torch.float32:
             return False
         c1, c2 = m.conv1, m.conv2
         if not isinstance(c2, BaseConv) or c2.conv.groups != 1 or c2.conv.kernel_size != (3, 3) or c2.conv.stride != (1, 1):
@@ -274,7 +271,7 @@ class Builder:
             return False
         if type(c1.act) is not type(c2.act) or len(x.segs) != 1 or x.segs[0] != c:
             return False
-        # c = 128 exists (bneck128_tc_kernel) but streams W2 through a 3-stage ring: 65 us vs 55 us for the unfused pair
+        # no fused kernel for c = 128: streaming W2 through a 3-stage ring measured 65 us vs 55 us for the unfused pair
         return c in (16, 32, 64)
 
     def bottleneck(self, x: Feat, m, out: Feat) -> Feat:
@@ -560,7 +557,7 @@ class InferenceEngine:
             self._post_ws = torch.empty((lib().yx_postprocess_workspace_bytes(batch, self.anchors),), dtype=torch.uint8,
                                         device=device)
             self.post = dict(post, max_det=max_det)
-            if self.dtype != torch.float32 and head.decode_in_inference and os.environ.get("YX_FUSED_FILTER", "1") != "0":
+            if self.dtype != torch.float32 and head.decode_in_inference:
                 cand, keys, counts = ops.postprocess_ws_ptrs(self._post_ws, batch, self.anchors)
                 self._post_fused = dict(cand=cand, keys=keys, counts=counts, conf_thre=post["conf_thre"])
                 b.postprocess_begin(self._post_ws, batch, self.anchors)

@@ -137,8 +137,7 @@ class BaseConv(_B200Block):
         y = conv2d(x, self.conv)             # tcgen05 forward / dgrad / wgrad under 16-bit autocast, else torch
         bn = self.bn
         if (y.is_cuda and bn.training and bn.momentum is not None and bn.track_running_stats and bn.affine
-                and bn.weight.dtype == torch.float32 and y.dim() == 4 and y.dtype in (torch.float32, torch.bfloat16, torch.float16)
-                and os.environ.get("YX_FUSED_BN", "1") != "0"):
+                and bn.weight.dtype == torch.float32 and y.dim() == 4 and y.dtype in (torch.float32, torch.bfloat16, torch.float16)):
             # nn.BatchNorm2d.forward in train mode: batch statistics, running statistics updated with `momentum`
             # (num_batches_tracked counts the calls), then the activation -- one fused pass each way
             # (num_batches_tracked counts the calls: incremented by the kernel)
@@ -230,7 +229,7 @@ class SPPBottleneck(_B200Block):
         from . import ops
 
         if (x.is_cuda and tuple(m.kernel_size for m in self.m) == (5, 9, 13) and x.dtype in (torch.bfloat16, torch.float16)
-                and ops._is_channels_last(x) and os.environ.get("YX_TRAIN_SPP", "1") != "0"):
+                and ops._is_channels_last(x)):
             x = _SppCat.apply(x)
         else:
             x = torch.cat([x] + [m(x) for m in self.m], dim=1)

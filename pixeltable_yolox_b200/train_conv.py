@@ -50,18 +50,18 @@ def direct_target(param: torch.Tensor) -> Optional[torch.Tensor]:
 
 
 # With direct gradient accumulation the weight-gradient launches have no consumer before the optimizer step, so they run on a
-# side streams (YX_WGRAD_STREAMS per device, round robin) next to the backward's critical chain  BatchNorm backward -> dgrad -> BatchNorm backward ...:
+# side streams (_N_WGRAD_STREAMS per device, round robin) next to the backward's critical chain  BatchNorm backward -> dgrad -> BatchNorm backward ...:
 # every kernel of an 8-image step is a fraction of a wave, so the two chains overlap (a CUDA-graph capture records the fork
 # and the join as graph branches). The wgrad inputs (saved activation, output gradient) are kept referenced until
 # `join_wgrad()` so that the caching allocator cannot hand their memory to the main stream while the side stream reads it.
 _wgrad_side = {}
 
 
-_N_WGRAD_STREAMS = max(1, int(os.environ.get("YX_WGRAD_STREAMS", "3")))
+_N_WGRAD_STREAMS = 3
 
 
 def _side(dev: torch.device):
-    """(stream, pending list) for the next weight gradient: round robin over YX_WGRAD_STREAMS side streams (each with its own
+    """(stream, pending list) for the next weight gradient: round robin over _N_WGRAD_STREAMS side streams (each with its own
     partial-sum workspace, ops.conv_wgrad keys it by stream), so consecutive layers' wgrad launches overlap each other too."""
     ent = _wgrad_side.get(dev)
     if ent is None:
@@ -205,7 +205,7 @@ class _ConvTc(torch.autograd.Function):
         xh = _pad_channels(x.detach().to(dtype), i_pad)
         # stride-2 dgrad: one sub-pixel conv over dy with a depth-to-space store when the input size is even, else the
         # rotated weights on the zero-stuffed dy
-        sub = stride == 2 and H % 2 == 0 and W % 2 == 0 and os.environ.get("YX_DGRAD_SUBPIXEL", "1") != "0"
+        sub = stride == 2 and H % 2 == 0 and W % 2 == 0
         pre = _packer.lookup(weight, dtype) if _packer is not None else None
         if pre is not None and (stride == 1 or sub):
             wf, wd = pre
@@ -233,14 +233,11 @@ class _ConvTc(torch.autograd.Function):
         if ctx.needs_input_grad[1]:
             target = direct_target(weight)
             if target is not None:
-                if os.environ.get("YX_WGRAD_OVERLAP", "1") != "0":
-                    stream, pending = _side(xh.device)
-                    stream.wait_event(torch.cuda.current_stream(xh.device).record_event())
-                    with torch.cuda.stream(stream):
-                        ops.conv_wgrad(xh, dyh, weight, k, stride, accumulate_into=target)
-                    pending.append((xh, dyh))
-                else:
+                stream, pending = _side(xh.device)
+                stream.wait_event(torch.cuda.current_stream(xh.device).record_event())
+                with torch.cuda.stream(stream):
                     ops.conv_wgrad(xh, dyh, weight, k, stride, accumulate_into=target)
+                pending.append((xh, dyh))
             else:
                 dw = ops.conv_wgrad(xh, dyh, weight, k, stride)
         if ctx.needs_input_grad[0]:

@@ -9,8 +9,6 @@ train : the network runs through PyTorch autograd; the SimOTA assignment of the 
 """
 from __future__ import annotations
 
-import os
-
 import math
 
 import torch
@@ -125,7 +123,7 @@ class YoloxHead(_B200Block):
             # the levels are independent chains (yolo_head.py:140-160): all but the last one (whose input is the final
             # neck op anyway) run as side lanes of the graph, forked right after the op that produced their input, so
             # the 80x80 chain overlaps the bottom-up half of the neck and the small 40x40 / 20x20 kernels
-            side = k < len(feats) - 1 and os.environ.get("YX_HEAD_LANES", "1") != "0"
+            side = k < len(feats) - 1
             if side:
                 b.begin_lane(k + 1, x)
             stem = self.stems[k].lower(b, x)

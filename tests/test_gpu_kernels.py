@@ -123,8 +123,8 @@ def _bneck_case(dev, B, H, W, c, dtype, use_add, act, in_off=0, out_off=0, seed=
 
 BNECK_CASES = [(2, 16, 16, 64), (1, 80, 80, 64), (3, 40, 40, 32), (1, 160, 160, 32), (2, 13, 21, 16), (1, 5, 3, 64),
                (5, 23, 61, 32), (2, 80, 80, 16)]
-# c = 128 (bneck128_tc_kernel, a measured regression: DESIGN 4.6) is only compiled into experiment builds
-BNECK128_CASES = [(2, 40, 40, 128), (1, 13, 21, 128), (9, 20, 20, 128), (1, 3, 5, 128)]
+# c = 128 has no fused kernel (a streamed-weight version measured slower than the unfused pair: DESIGN 4.6)
+C128_CASES = [(2, 40, 40, 128), (1, 13, 21, 128), (9, 20, 20, 128), (1, 3, 5, 128)]
 
 
 @pytest.mark.parametrize("case", BNECK_CASES)
@@ -138,15 +138,10 @@ def test_fused_bottleneck_vs_torch(cuda, case, dtype):
         assert err <= tol, (use_add, err)
 
 
-@pytest.mark.parametrize("case", BNECK128_CASES)
-def test_fused_bottleneck_128_experiment_build_only(cuda, case):
-    import os
-
-    if "exp" not in os.environ.get("YX_B200_LIB", ""):
-        with pytest.raises(RuntimeError, match="16, 32 or 64"):
-            _bneck_case(cuda, *case, torch.bfloat16, True, "silu")
-        return
-    assert _bneck_case(cuda, *case, torch.bfloat16, True, "silu") <= 2e-2
+@pytest.mark.parametrize("case", C128_CASES)
+def test_fused_bottleneck_rejects_c128(cuda, case):
+    with pytest.raises(RuntimeError, match="16, 32 or 64"):
+        _bneck_case(cuda, *case, torch.bfloat16, True, "silu")
 
 
 def test_fused_bottleneck_slices_and_acts(cuda):

@@ -48,7 +48,6 @@ def _no_tf32():
 
 
 def _set_ctas(monkeypatch, ctas):
-    monkeypatch.delenv("YX_CTAS_MAXPIX", raising=False)
     if ctas is None:
         monkeypatch.delenv("YX_CTAS_PER_SM", raising=False)
     else:

@@ -47,21 +47,7 @@ def all_kept(batch, classes):
 
 
 rows = []
-PHASES_ONLY = "--phases-only" in sys.argv
-if "--flush-sweep" in sys.argv:
-    # batch rows at which a survivor batch is resolved (YX_NMS_FLUSH): time + equality of the kept rows against the default
-    dense = torch.from_numpy(syn.dense_scene(64, anchors=A, seed=13)).to(dev)
-    for thr in (0.001, 0.25, 0.5):
-        base_t, base_o = timed(dense, thr)
-        cnt = base_o[2].cpu().tolist()
-        for fl in ("128", "192", "256", "320", "384", "448", "512"):
-            os.environ["YX_NMS_FLUSH"] = fl
-            t, o = timed(dense, thr)
-            del os.environ["YX_NMS_FLUSH"]
-            same = bool(torch.equal(o[2], base_o[2])) and all(bool(torch.equal(o[1][b, :cnt[b]], base_o[1][b, :cnt[b]])) for b in range(64))
-            print(json.dumps(dict(conf_thre=thr, flush_rows=int(fl), postprocess_us=round(t, 1), default_us=round(base_t, 1), rows_equal=same)), flush=True)
-    sys.exit(0)
-for batch in (() if PHASES_ONLY else (64, 16, 4, 1)):
+for batch in (64, 16, 4, 1):
     dense = torch.from_numpy(syn.dense_scene(batch, anchors=A, seed=13)).to(dev)
     kept3 = torch.from_numpy(all_kept(batch, 3)).to(dev)
     for name, pred, thr in (("dense", dense, 0.001), ("dense", dense, 0.25), ("dense", dense, 0.5), ("all_kept_3_classes", kept3, 0.01)):
@@ -77,19 +63,6 @@ for batch in (() if PHASES_ONLY else (64, 16, 4, 1)):
                    postprocess_us_cluster=round(tc, 1), speedup=round(t1 / tc, 2), rows_equal=same)
         print(json.dumps(row), flush=True)
         rows.append(row)
-for batch in (64, 1):
-    dense = torch.from_numpy(syn.dense_scene(batch, anchors=A, seed=13)).to(dev)
-    for cap in ("1", "2", None):
-        if cap:
-            os.environ["YX_NMS_CLUSTER"] = cap
-        ops.postprocess_device(dense.clone(), 80, 0.001, 0.65, NMS_VARIANTS["auto"])
-        torch.cuda.synchronize()
-        os.environ["YX_NMS_DEBUG"] = "1"
-        print(f"== phases (clk), batch {batch}, cluster cap {cap or 'auto'}: dense thr 0.001", flush=True)
-        ops.postprocess_device(dense.clone(), 80, 0.001, 0.65, NMS_VARIANTS["auto"])
-        torch.cuda.synchronize()
-        del os.environ["YX_NMS_DEBUG"]
-        os.environ.pop("YX_NMS_CLUSTER", None)
-if len(sys.argv) > 1 and not PHASES_ONLY:
+if len(sys.argv) > 1:
     Path(sys.argv[1]).write_text(json.dumps(rows, indent=1))
 assert all(r["rows_equal"] for r in rows), "cluster kernel keeps different rows"

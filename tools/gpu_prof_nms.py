@@ -1,7 +1,6 @@
 """Device time of the sort + NMS kernel (yx_nms_prefiltered after one filter pass) and of the score filter on
 B = 64 images: sparse scenes (~20 candidates, the bench's regime: single-warp path), dense scenes at three thresholds
 (config 5) and the degenerate every-anchor-kept scene (conf 0.01 on random weights). CUDA-graph replay, no Python time."""
-import os
 import sys
 from pathlib import Path
 
@@ -57,5 +56,3 @@ rng = np.random.default_rng(10)
 grid[:, :, 4] = rng.uniform(0.5, 1.0, (B, A))
 np.put_along_axis(grid[:, :, 5:], rng.integers(0, 80, (B, A))[..., None], 0.9, axis=2)
 case("every anchor kept (disjoint)", grid, 0.01)
-if os.environ.get("YX_NMS_DEBUG"):
-    pass

@@ -20,13 +20,15 @@ H = {}
 
 
 def walk():
-    # BN shapes = BaseConv outputs: run the torch train forward on the meta device
+    # BN shapes = outputs of the convs inside BaseConv: run the train forward with the convs on torch, whose hooks fire
+    from pixeltable_yolox_b200.network_blocks import BaseConv
+
     def hook(m, inp, out):
         key = tuple(out.shape[1:])
         shapes[key] = shapes.get(key, 0) + 1
-    hs = [m.register_forward_hook(hook) for m in model.modules() if isinstance(m, torch.nn.BatchNorm2d)]
+    hs = [m.conv.register_forward_hook(hook) for m in model.modules() if isinstance(m, BaseConv)]
     import os
-    os.environ["YX_TRAIN_CONV"] = "0"; os.environ["YX_FUSED_BN"] = "0"
+    os.environ["YX_TRAIN_CONV"] = "0"
     model.to(dev).train()
     with torch.no_grad():
         lab = torch.zeros(1, 120, 5, device=dev); lab[:, 0] = torch.tensor([1.0, 320, 320, 100, 100], device=dev)

@@ -43,5 +43,5 @@ for seed in range(seeds):
     rows.append((cos(res["ours"][1], g32), cos(res["torch16"][1], g32), abs(res["ours"][0] - l32) / l32, abs(res["torch16"][0] - l32) / l32))
     print(f"seed {seed}: gradient cosine vs fp32 ours {rows[-1][0]:.4f} torch16 {rows[-1][1]:.4f} | loss rel err ours {rows[-1][2]:.2e} torch16 {rows[-1][3]:.2e}", flush=True)
 n = len(rows)
-print(f"mean over {n} seeds (YX_BN_PRECISE={os.environ.get('YX_BN_PRECISE', '0')}): cosine ours {sum(r[0] for r in rows) / n:.4f} torch16 {sum(r[1] for r in rows) / n:.4f} | "
+print(f"mean over {n} seeds: cosine ours {sum(r[0] for r in rows) / n:.4f} torch16 {sum(r[1] for r in rows) / n:.4f} | "
       f"loss rel err ours {sum(r[2] for r in rows) / n:.2e} torch16 {sum(r[3] for r in rows) / n:.2e}")
