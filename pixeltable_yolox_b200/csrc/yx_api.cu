@@ -127,6 +127,45 @@ int num_sms() {
   return cached;
 }
 
+int max_smem_optin() {
+  static int cached_dev[kMaxDevices] = {};
+  int& cached = cached_dev[current_device_slot()];
+  if (!cached) {
+    int dev = 0, n = 0;
+    if (cudaGetDevice(&dev) == cudaSuccess &&
+        cudaDeviceGetAttribute(&n, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) == cudaSuccess && n > 0)
+      cached = n;
+  }
+  return cached;
+}
+
+int encode_tma(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims,
+               const cuuint64_t* byte_strides, const cuuint32_t* box, const cuuint32_t* elem_strides,
+               CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* what) {
+  // a driver entry point: resolved through the runtime, so the library loads without libcuda
+  static const auto encode = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                    q == cudaDriverEntryPointSuccess;
+    return reinterpret_cast<decltype(&cuTensorMapEncodeTiled)>(ok ? p : nullptr);
+  }();
+  YX_REQUIRE(encode != nullptr, YX_ERR_NO_DEVICE, "cuTensorMapEncodeTiled unavailable (no CUDA driver)");
+  static const cuuint32_t ones[5] = {1, 1, 1, 1, 1};
+  const CUresult r = encode(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, byte_strides, box,
+                            elem_strides ? elem_strides : ones, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2,
+                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char shape[192];   // rank <= 5: " size/box" fits 32 characters per dimension
+    int n = 0;
+    for (int i = 0; i < rank; ++i) n += snprintf(shape + n, sizeof(shape) - n, " %llu/%u", (unsigned long long)dims[i], box[i]);
+    set_error("cuTensorMapEncodeTiled(%s) failed: %d (size/box per dimension:%s; row pitch %llu bytes)", what, (int)r, shape,
+              rank > 1 ? (unsigned long long)byte_strides[0] : 0ull);
+    return YX_ERR_CUDA;
+  }
+  return YX_OK;
+}
+
 static int require_device() {
   static int ok_dev[kMaxDevices] = {};         // checked once per device, not once per process
   int& ok = ok_dev[current_device_slot()];
@@ -242,6 +281,7 @@ int yx_conv_bn_act_fwd(const yx_conv_desc* d, void* stream) {
   YX_REQUIRE(d != nullptr, YX_ERR_INVALID_ARG, "conv: null descriptor");
   if (d->dtype == YX_FP32) return conv_simt_launch(d, (cudaStream_t)stream);
   ConvTcLaunch* L = conv_tc_alloc();
+  YX_REQUIRE(L != nullptr, YX_ERR_INVALID_ARG, "conv: out of host memory");
   rc = conv_tc_prepare(d, L);
   if (rc == YX_OK) rc = conv_tc_launch(L, (cudaStream_t)stream);
   conv_tc_free(L);
@@ -262,6 +302,7 @@ int yx_bottleneck_fwd(const yx_bneck_desc* d, void* stream) {
   int rc = require_device();
   if (rc) return rc;
   BneckLaunch* L = bneck_alloc();
+  YX_REQUIRE(L != nullptr, YX_ERR_INVALID_ARG, "bottleneck: out of host memory");
   rc = bneck_prepare(d, L);
   if (rc == YX_OK) rc = bneck_launch(L, (cudaStream_t)stream);
   bneck_free(L);
@@ -301,6 +342,7 @@ int yx_focus_conv_bn_act_fwd(const void* img, int32_t img_dtype, const void* w, 
   int rc = require_device();
   if (rc) return rc;
   StemLaunch* L = stem_alloc();
+  YX_REQUIRE(L != nullptr, YX_ERR_INVALID_ARG, "stem: out of host memory");
   rc = stem_prepare(img, img_dtype, w, bias, out, out_ld, batch, h, wd, out_c, act, dtype, L);
   if (rc == YX_OK) rc = stem_launch(L, (cudaStream_t)stream);
   stem_free(L);
@@ -580,6 +622,7 @@ int yx_plan_add_conv(yx_plan* p, const yx_conv_desc* d) {
   } else {
     o.kind = OP_CONV_TC;
     o.tc = conv_tc_alloc();
+    YX_REQUIRE(o.tc != nullptr, YX_ERR_INVALID_ARG, "plan_add_conv: out of host memory");
     rc = conv_tc_prepare(d, o.tc);
     if (rc) { conv_tc_free(o.tc); return rc; }
   }
@@ -597,6 +640,7 @@ int yx_plan_add_bottleneck(yx_plan* p, const yx_bneck_desc* d) {
   memset(&o, 0, sizeof(o));
   o.kind = OP_BNECK;
   o.bneck = bneck_alloc();
+  YX_REQUIRE(o.bneck != nullptr, YX_ERR_INVALID_ARG, "plan_add_bottleneck: out of host memory");
   rc = bneck_prepare(d, o.bneck);
   if (rc) { bneck_free(o.bneck); return rc; }
   plan_push(p, o);
@@ -654,6 +698,7 @@ int yx_plan_add_focus_conv(yx_plan* p, const void* img, int32_t img_dtype, const
   memset(&o, 0, sizeof(o));
   o.kind = OP_STEM;
   o.stem = stem_alloc();
+  YX_REQUIRE(o.stem != nullptr, YX_ERR_INVALID_ARG, "plan_add_focus_conv: out of host memory");
   rc = stem_prepare(img, img_dtype, w, bias, out, out_ld, batch, h, wd, out_c, act, dtype, o.stem);
   if (rc) { stem_free(o.stem); return rc; }
   plan_push(p, o);

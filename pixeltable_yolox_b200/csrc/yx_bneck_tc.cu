@@ -17,8 +17,9 @@
 // per SM walks a contiguous range of tiles; GEMM1 of tile i+1 is issued before GEMM2 of tile i so
 // the two epilogue groups and the tensor core overlap. Channels: C in {16, 32, 64} (one swizzle row).
 // HBM traffic per pixel: C in + C out (the unfused pair moves 5 C with the shortcut).
-#include <stdlib.h>
 #include <string.h>
+
+#include <new>
 
 #include "yx_tc_epilogue.cuh"
 
@@ -353,12 +354,6 @@ bneck_tc_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 struct BneckLaunch {
   CUtensorMap map_x, map_w1, map_w2;
   BneckParams p;
@@ -366,13 +361,8 @@ struct BneckLaunch {
   size_t smem;
 };
 
-BneckLaunch* bneck_alloc() {
-  void* p = nullptr;
-  if (posix_memalign(&p, 64, sizeof(BneckLaunch)) != 0) return nullptr;
-  memset(p, 0, sizeof(BneckLaunch));
-  return reinterpret_cast<BneckLaunch*>(p);
-}
-void bneck_free(BneckLaunch* p) { free(p); }
+BneckLaunch* bneck_alloc() { return new (std::nothrow) BneckLaunch(); }
+void bneck_free(BneckLaunch* p) { delete p; }
 
 bool bneck_supported(const yx_bneck_desc* d) {
   return d && (d->c == 16 || d->c == 32 || d->c == 64) && (d->dtype == YX_BF16 || d->dtype == YX_FP16);
@@ -404,8 +394,6 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
     }
     YX_REQUIRE(ok, YX_ERR_INVALID_ARG, "bottleneck: out must not alias x (the fused kernel cannot run in place)");
   }
-  EncodeTiledFn encode = get_encode_fn();
-  YX_REQUIRE(encode != nullptr, YX_ERR_NO_DEVICE, "cuTensorMapEncodeTiled unavailable (no CUDA driver)");
   BneckParams& p = L->p;
   memset(&p, 0, sizeof(p));
   p.C = d->c; p.Cpad = d->c < 32 ? 32 : d->c;
@@ -439,81 +427,59 @@ int bneck_prepare(const yx_bneck_desc* d, BneckLaunch* L) {
   p.w_tx_bytes = (unsigned)d->c * p.row_bytes;
   p.bias_bytes = 1024u;
   p.tmem_cols = 32; while (p.tmem_cols < (unsigned)(6 * p.Cpad)) p.tmem_cols <<= 1;
-  const unsigned layout = d->c == 64 ? 2u : (d->c == 32 ? 4u : 6u);
-  p.desc_hi = (((8u * p.row_bytes) >> 4) & 0x3FFFu) | (1u << 14) | (layout << 29);
-  const unsigned fmt = d->dtype == YX_BF16 ? 1u : 0u;
-  p.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((unsigned)(d->c >> 3) << 17) | ((128u >> 4) << 24);
+  p.desc_hi = umma_desc_hi(p.row_bytes);
+  p.idesc = umma_idesc(d->dtype, d->c);
   p.act1 = d->act; p.bias1 = d->bias1;
   EpiParams& e = p.epi;
   e.out_h = d->h; e.out_w = d->w; e.out_c = d->c; e.act = d->act; e.dtype = d->dtype; e.epilogue = YX_EPI_STORE;
   e.bias = d->bias2; e.out = d->out; e.out_ld = d->out_ld;
   e.res = d->use_add ? d->x : nullptr; e.res_ld = d->x_ld;
-  int dev = 0, max_smem = 0;
-  YX_CUDA(cudaGetDevice(&dev));
-  YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  const int max_smem = max_smem_optin();
   const long long fixed = 2048 + 2 * (long long)p.bias_bytes + 2 * (long long)p.h_slot_bytes + 10 * (long long)p.w_tile_bytes;
   p.nx = (int)((max_smem - fixed) / p.x_slot_bytes);
   if (p.nx > kBnX) p.nx = kBnX;
   YX_REQUIRE(p.nx >= 2, YX_ERR_UNSUPPORTED, "bottleneck: shared memory too small (%lld fixed bytes)", fixed);
   L->smem = (size_t)fixed + (size_t)p.nx * p.x_slot_bytes;
 
-  const CUtensorMapDataType tdt = d->dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  const CUtensorMapSwizzle sw = d->c == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (d->c == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+  const CUtensorMapDataType tdt = tma_dtype(d->dtype);
+  const CUtensorMapSwizzle sw = tma_swizzle(p.row_bytes);
   {
     cuuint64_t dims[4] = {(cuuint64_t)d->c, (cuuint64_t)d->w, (cuuint64_t)d->h, (cuuint64_t)d->batch};
     cuuint64_t strides[3] = {(cuuint64_t)d->x_ld * 2, (cuuint64_t)d->x_ld * 2 * d->w, (cuuint64_t)d->x_ld * 2 * d->w * d->h};
     cuuint32_t box[4] = {(cuuint32_t)d->c, (cuuint32_t)p.pitch, (cuuint32_t)(p.th + 2), 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->map_x, tdt, 4, const_cast<void*>(d->x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                        CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(bottleneck x) failed: %d", (int)r);
+    const int rc = encode_tma(&L->map_x, tdt, 4, d->x, dims, strides, box, nullptr, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                              "bottleneck x");
+    if (rc) return rc;
   }
   for (int which = 0; which < 2; ++which) {
     const cuuint64_t K = (cuuint64_t)(which ? 9 : 1) * d->c;
     cuuint64_t dims[2] = {K, (cuuint64_t)d->c};
     cuuint64_t strides[1] = {K * 2};
     cuuint32_t box[2] = {(cuuint32_t)d->c, (cuuint32_t)d->c};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(which ? &L->map_w2 : &L->map_w1, tdt, 2, const_cast<void*>(which ? d->w2 : d->w1), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(bottleneck W%d) failed: %d", which + 1, (int)r);
+    const int rc = encode_tma(which ? &L->map_w2 : &L->map_w1, tdt, 2, which ? d->w2 : d->w1, dims, strides, box, nullptr, sw,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, which ? "bottleneck W2" : "bottleneck W1");
+    if (rc) return rc;
   }
   const int sms = num_sms();
   L->grid = p.num_tiles < sms ? p.num_tiles : sms;
   return YX_OK;
 }
 
+// [fp16][KS = 1, 2, 4][SiLU]
+static decltype(&bneck_tc_kernel<false, 1, false>) const kBneckKernels[2][3][2] = {
+    {{bneck_tc_kernel<false, 1, false>, bneck_tc_kernel<false, 1, true>},
+     {bneck_tc_kernel<false, 2, false>, bneck_tc_kernel<false, 2, true>},
+     {bneck_tc_kernel<false, 4, false>, bneck_tc_kernel<false, 4, true>}},
+    {{bneck_tc_kernel<true, 1, false>, bneck_tc_kernel<true, 1, true>},
+     {bneck_tc_kernel<true, 2, false>, bneck_tc_kernel<true, 2, true>},
+     {bneck_tc_kernel<true, 4, false>, bneck_tc_kernel<true, 4, true>}}};
+
 int bneck_launch(const BneckLaunch* L, cudaStream_t stream) {
-  static bool attr_set_dev[kMaxDevices] = {};
-  bool& attr_set = attr_set_dev[current_device_slot()];
-  if (!attr_set) {
-    int dev = 0, max_smem = 0;
-    YX_CUDA(cudaGetDevice(&dev));
-    YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-#define YX_BN_ATTR(F, K) YX_CUDA(cudaFuncSetAttribute(bneck_tc_kernel<F, K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem)); \
-  YX_CUDA(cudaFuncSetAttribute(bneck_tc_kernel<F, K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem))
-    YX_BN_ATTR(false, 1); YX_BN_ATTR(false, 2); YX_BN_ATTR(false, 4); YX_BN_ATTR(true, 1); YX_BN_ATTR(true, 2); YX_BN_ATTR(true, 4);
-#undef YX_BN_ATTR
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)L->grid);
-  cfg.blockDim = dim3((unsigned)kBnThreads);
-  cfg.dynamicSmemBytes = L->smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const bool h16 = L->p.epi.dtype == YX_FP16;
-#define YX_BN_GO(F, K) do { if (L->p.act1 == YX_ACT_SILU) YX_CUDA(cudaLaunchKernelEx(&cfg, bneck_tc_kernel<F, K, true>, L->map_x, L->map_w1, L->map_w2, L->p)); \
-    else YX_CUDA(cudaLaunchKernelEx(&cfg, bneck_tc_kernel<F, K, false>, L->map_x, L->map_w1, L->map_w2, L->p)); } while (0)
-  if (L->p.ksteps == 4) { if (h16) YX_BN_GO(true, 4); else YX_BN_GO(false, 4); }
-  else if (L->p.ksteps == 2) { if (h16) YX_BN_GO(true, 2); else YX_BN_GO(false, 2); }
-  else { if (h16) YX_BN_GO(true, 1); else YX_BN_GO(false, 1); }
-#undef YX_BN_GO
+  static bool smem_set[kMaxDevices] = {};
+  YX_CUDA(opt_in_smem(smem_set, kBneckKernels, [](int) { return max_smem_optin(); }));
+  const auto kernel = kBneckKernels[L->p.epi.dtype == YX_FP16][L->p.ksteps / 2][L->p.act1 == YX_ACT_SILU];
+  YX_CUDA(launch_pdl(kernel, dim3((unsigned)L->grid), dim3((unsigned)kBnThreads), L->smem, stream, L->map_x, L->map_w1, L->map_w2,
+                     L->p));
   return YX_OK;
 }
 

@@ -1,5 +1,5 @@
-// Shared device/host helpers for the sm_100a YOLOX kernels: error plumbing, PTX wrappers for
-// mbarrier / TMA / tcgen05 / TMEM, and small numeric helpers.
+// Shared device/host helpers for the sm_100a YOLOX kernels: error plumbing, TMA maps, tcgen05 descriptor
+// formats and launches, PTX wrappers for mbarrier / TMA / tcgen05 / TMEM, and small numeric helpers.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -7,6 +7,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+
+#include <type_traits>
 
 #include "../../include/yx_b200.h"
 
@@ -46,6 +48,44 @@ int num_sms();  // SM count of the current device (cached)
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline int dtype_size(int dt) { return dt == YX_FP32 ? 4 : (dt == YX_U8 ? 1 : 2); }
 
+// ------------------------------------------------------------------------------------------
+// host side: tcgen05 operand formats and TMA tensor maps
+// ------------------------------------------------------------------------------------------
+int max_smem_optin();  // opt-in shared memory per block of the current device (cached; 0 if it cannot be queried)
+
+// Encodes a tiled TMA map (no interleave, zero fill out of bounds); elem_strides == nullptr means all 1. Returns YX_OK,
+// YX_ERR_NO_DEVICE without a driver entry point, or YX_ERR_CUDA with an error message naming `what` and the shape.
+int encode_tma(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims,
+               const cuuint64_t* byte_strides, const cuuint32_t* box, const cuuint32_t* elem_strides,
+               CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* what);
+
+inline CUtensorMapDataType tma_dtype(int dt) {
+  switch (dt) {
+    case YX_BF16: return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    case YX_FP16: return CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    case YX_FP32: return CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    default: return CU_TENSOR_MAP_DATA_TYPE_UINT8;
+  }
+}
+
+// Operand rows of 32, 64 or 128 bytes (16, 32 or 64 16-bit channels) are stored with the swizzle of the same span: TMA writes
+// that layout with tma_swizzle(row_bytes) and the UMMA descriptor names it by layout type 6, 4 or 2.
+inline CUtensorMapSwizzle tma_swizzle(unsigned row_bytes) {
+  return row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+}
+// Upper word of the UMMA shared-memory descriptor: stride byte offset = one 8-row atom (>> 4), version 1, layout type
+inline unsigned umma_desc_hi(unsigned row_bytes) {
+  const unsigned layout = row_bytes == 128 ? 2u : (row_bytes == 64 ? 4u : 6u);
+  return (((8u * row_bytes) >> 4) & 0x3FFFu) | (1u << 14) | (layout << 29);
+}
+// UMMA instruction descriptor of a kind::f16 MMA, M = 128, N = n: fp32 accumulate, A and B in `dtype` (bf16 or fp16),
+// both K-major, or both MN-major (bits 15, 16)
+inline unsigned umma_idesc(int dtype, int n, bool mn_major = false) {
+  const unsigned fmt = dtype == YX_BF16 ? 1u : 0u;
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | (mn_major ? (1u << 15) | (1u << 16) : 0u) | ((unsigned)(n >> 3) << 17) |
+         ((128u >> 4) << 24);
+}
+
 #ifdef __CUDACC__
 // Plain launch that returns the launch error. The training step's chains of small kernels (BatchNorm, wgrad, packing) do
 // not use programmatic dependent launch: it measured slower than plain launches there (9.32 vs 8.70 ms per step, 8 images).
@@ -54,6 +94,37 @@ inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
   return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
+// launch_kernel with programmatic dependent launch: the kernel's prologue may overlap the tail of its predecessor in the
+// stream; the kernel waits for the predecessor's writes with pdl_wait().
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
+  cudaLaunchAttribute pdl = {};
+  pdl.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  pdl.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+  cfg.attrs = &pdl; cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
+// Raises the dynamic shared-memory limit of every kernel in `kernels` (one kernel pointer or an array of them of any rank)
+// to smem_bytes(i) for the i-th in row-major order. Kernel attributes belong to a device: this happens on the first call on
+// each device, `done` holding the table's per-device flags. Later calls make no CUDA runtime call besides the device lookup,
+// so launches inside a CUDA-graph capture may make them; smem_bytes is evaluated on the first call only.
+template <typename Table, typename Bytes>
+inline cudaError_t opt_in_smem(bool (&done)[kMaxDevices], const Table& kernels, Bytes smem_bytes) {
+  bool& d = done[current_device_slot()];
+  if (d) return cudaSuccess;
+  using Kernel = typename std::remove_all_extents<Table>::type;
+  const Kernel* k = reinterpret_cast<const Kernel*>(&kernels);
+  for (int i = 0; i < (int)(sizeof(Table) / sizeof(Kernel)); ++i) {
+    const cudaError_t e = cudaFuncSetAttribute(k[i], cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(i));
+    if (e != cudaSuccess) return e;
+  }
+  d = true;
+  return cudaSuccess;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -24,6 +24,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <new>
+
 #include "yx_tc_epilogue.cuh"
 
 namespace yx {
@@ -782,25 +784,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
 struct ConvTcLaunch {
   CUtensorMap map_a, map_b;
   ConvTcParams p;
@@ -916,8 +899,6 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   memset(&p, 0, sizeof(p));
   rc = fill_epi_params(d, &p.epi);
   if (rc) return rc;
-  EncodeTiledFn encode = get_encode_fn();
-  YX_REQUIRE(encode != nullptr, YX_ERR_NO_DEVICE, "cuTensorMapEncodeTiled unavailable (no CUDA driver)");
 
   p.ksize = d->ksize; p.stride = d->stride; p.pad = (d->ksize - 1) / 2;
   p.in_c = d->in_c; p.batch = d->batch;
@@ -950,9 +931,7 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   const unsigned row_bytes = (unsigned)p.KC * 2;             // 128 / 64 / 32 = swizzle span
   p.row_bytes = row_bytes;
   p.G = 1; p.a_slots = 0; p.b_region_bytes = 0;
-  int dev = 0, max_smem = 0;
-  YX_CUDA(cudaGetDevice(&dev));
-  YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  int max_smem = max_smem_optin();
   if (ctas == 2 && max_smem > 112 * 1024) max_smem = 112 * 1024;       // 228 KB per SM, 1 KB reserved per CTA
   p.bias_bytes = ((unsigned)d->out_c * 4u + 1023u) & ~1023u;
 
@@ -1111,16 +1090,10 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
   L->smem = fixed_bytes + (size_t)stages * p.stage_bytes;
   }
 
-  // UMMA shared-memory descriptor, upper word: SBO = 8 rows * row_bytes, version 1, layout type
-  const unsigned layout = p.KC == 64 ? 2u : (p.KC == 32 ? 4u : 6u);  // SW128 / SW64 / SW32
-  const unsigned sbo = (8u * row_bytes) >> 4;
-  p.desc_hi = (sbo & 0x3FFFu) | (1u << 14) | (layout << 29);
-  const unsigned fmt = d->dtype == YX_BF16 ? 1u : 0u;
-  p.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((unsigned)(p.BN >> 3) << 17) | ((128u >> 4) << 24);
-
-  const CUtensorMapDataType tdt = d->dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  const CUtensorMapSwizzle sw = p.KC == 64 ? CU_TENSOR_MAP_SWIZZLE_128B
-                               : (p.KC == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+  p.desc_hi = umma_desc_hi(row_bytes);
+  p.idesc = umma_idesc(d->dtype, p.BN);
+  const CUtensorMapDataType tdt = tma_dtype(d->dtype);
+  const CUtensorMapSwizzle sw = tma_swizzle(row_bytes);
   {
     cuuint64_t dims[4], strides[3];
     cuuint32_t box[4], estr[4];
@@ -1146,22 +1119,16 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
         estr[1] = 1;
       }
     }
-    CUresult r = encode(&L->map_a, tdt, 4, const_cast<void*>(d->in), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(A) failed: %d (in_c=%d ld=%lld box=%u,%u,%u)",
-               (int)r, d->in_c, (long long)d->in_ld, box[0], box[1], box[2]);
+    rc = encode_tma(&L->map_a, tdt, 4, d->in, dims, strides, box, estr, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "A");
+    if (rc) return rc;
   }
   {
     const cuuint64_t K = (cuuint64_t)d->ksize * d->ksize * d->in_c;
     cuuint64_t dims[2] = {K, (cuuint64_t)d->out_c};
     cuuint64_t strides[1] = {K * 2};
     cuuint32_t box[2] = {(cuuint32_t)p.KC, (cuuint32_t)p.BN};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(&L->map_b, tdt, 2, const_cast<void*>(d->w), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(W) failed: %d", (int)r);
+    rc = encode_tma(&L->map_b, tdt, 2, d->w, dims, strides, box, nullptr, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "W");
+    if (rc) return rc;
   }
   p.mul_tpi = fast_div_mul(p.tiles_w * p.tiles_h);
   p.mul_tw = fast_div_mul(p.tiles_w);
@@ -1180,68 +1147,36 @@ static int conv_tc_prepare_mode(const yx_conv_desc* d, ConvTcLaunch* L, bool all
 
 int conv_tc_prepare(const yx_conv_desc* d, ConvTcLaunch* L) { return conv_tc_prepare_mode(d, L, true); }
 
-ConvTcLaunch* conv_tc_alloc() {
-  void* p = nullptr;
-  if (posix_memalign(&p, 64, sizeof(ConvTcLaunch)) != 0) return nullptr;  // CUtensorMap wants 64-byte alignment
-  memset(p, 0, sizeof(ConvTcLaunch));
-  return reinterpret_cast<ConvTcLaunch*>(p);
-}
-void conv_tc_free(ConvTcLaunch* p) { free(p); }
+ConvTcLaunch* conv_tc_alloc() { return new (std::nothrow) ConvTcLaunch(); }
+void conv_tc_free(ConvTcLaunch* p) { delete p; }
 
 // The launch selection of conv_tc_prepare, without a launch (yx_conv_schedule): tests use it to show which mode, ring
 // depths and per-CTA tile ranges a shape exercises.
 int conv_tc_schedule(const yx_conv_desc* d, int32_t* info, int capacity) {
-  ConvTcLaunch* L = conv_tc_alloc();
-  YX_REQUIRE(L != nullptr, YX_ERR_INVALID_ARG, "conv_schedule: out of host memory");
-  const int rc = conv_tc_prepare(d, L);
+  ConvTcLaunch L = {};
+  const int rc = conv_tc_prepare(d, &L);
+  if (rc) return rc;
+  const ConvTcParams& p = L.p;
+  const int32_t v[] = {p.halo, p.flat, p.b_resident, p.G, L.ctas, p.epi_groups, p.acc_stages, p.a_slots,
+                       p.stages, p.BN, p.n_tiles, p.m_tiles, p.num_tiles, L.grid, p.tw, p.th};
   int n = 0;
-  if (rc == YX_OK) {
-    const ConvTcParams& p = L->p;
-    const int32_t v[] = {p.halo, p.flat, p.b_resident, p.G, L->ctas, p.epi_groups, p.acc_stages, p.a_slots,
-                         p.stages, p.BN, p.n_tiles, p.m_tiles, p.num_tiles, L->grid, p.tw, p.th};
-    for (; n < (int)(sizeof(v) / sizeof(v[0])) && n < capacity; ++n) info[n] = v[n];
-  }
-  conv_tc_free(L);
-  return rc == YX_OK ? n : rc;
+  for (; n < (int)(sizeof(v) / sizeof(v[0])) && n < capacity; ++n) info[n] = v[n];
+  return n;
 }
 
+// [fp16][store, store + SiLU, head]: the head epilogue has no SiLU instantiation
+static decltype(&conv_tc_kernel<false, false, false>) const kConvKernels[2][3] = {
+    {conv_tc_kernel<false, false, false>, conv_tc_kernel<false, true, false>, conv_tc_kernel<false, false, true>},
+    {conv_tc_kernel<true, false, false>, conv_tc_kernel<true, true, false>, conv_tc_kernel<true, false, true>}};
+
 int conv_tc_launch(const ConvTcLaunch* L, cudaStream_t stream) {
-  static bool attr_set_dev[kMaxDevices] = {};
-  bool& attr_set = attr_set_dev[current_device_slot()];
-  if (!attr_set) {
-    int dev = 0, max_smem = 0;
-    YX_CUDA(cudaGetDevice(&dev));
-    YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    YX_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)L->grid);
-  cfg.blockDim = dim3((unsigned)(64 + 128 * L->p.epi_groups));
-  cfg.dynamicSmemBytes = L->smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const bool silu = L->p.epi.act == YX_ACT_SILU && L->p.epi.epilogue == YX_EPI_STORE;
-  const bool head = L->p.epi.epilogue == YX_EPI_HEAD;
-  if (L->p.epi.dtype == YX_FP16) {
-    if (head) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, true>, L->map_a, L->map_b, L->p));
-    else if (silu) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, true, false>, L->map_a, L->map_b, L->p));
-    else YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<true, false, false>, L->map_a, L->map_b, L->p));
-  } else {
-    if (head) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, true>, L->map_a, L->map_b, L->p));
-    else if (silu) YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, true, false>, L->map_a, L->map_b, L->p));
-    else YX_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<false, false, false>, L->map_a, L->map_b, L->p));
-  }
+  static bool smem_set[kMaxDevices] = {};
+  YX_CUDA(opt_in_smem(smem_set, kConvKernels, [](int) { return max_smem_optin(); }));
+  const EpiParams& e = L->p.epi;
+  const int epi = e.epilogue == YX_EPI_HEAD ? 2 : (e.act == YX_ACT_SILU ? 1 : 0);
+  const auto kernel = kConvKernels[e.dtype == YX_FP16][epi];
+  YX_CUDA(launch_pdl(kernel, dim3((unsigned)L->grid), dim3((unsigned)(64 + 128 * L->p.epi_groups)), L->smem, stream, L->map_a,
+                     L->map_b, L->p));
   return YX_OK;
 }
 

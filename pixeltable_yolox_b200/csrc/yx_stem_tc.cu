@@ -19,8 +19,9 @@
 //   warps 10-17 two epilogue groups (bias + SiLU + 256-bit stores).
 // K order inside a tap: k = 2*(2*c + py) + px for image channel c and pixel parity (py, px), i.e. Focus channel
 // 3*(2*px + py) + c (network_blocks.py:199-207: TL, BL, TR, BR); k = 12..15 are zero.
-#include <stdlib.h>
 #include <string.h>
+
+#include <new>
 
 #include "yx_tc_epilogue.cuh"
 
@@ -324,12 +325,6 @@ stem_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant_
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();
-
 struct StemLaunch {
   CUtensorMap map_w, map_img;
   StemParams p;
@@ -343,13 +338,8 @@ struct StemLaunch {
 // the kernel is not latency-bound after all: ncu (profiles/r2_stem.md) has the L1 data pipe saturated -- LSU wavefronts 68 %
 // (shared loads of the builders and epilogues 39 %, stores 9 %) + tensor-core operand reads 34 % of the same pipe.
 
-StemLaunch* stem_alloc() {
-  void* p = nullptr;
-  if (posix_memalign(&p, 64, sizeof(StemLaunch)) != 0) return nullptr;
-  memset(p, 0, sizeof(StemLaunch));
-  return reinterpret_cast<StemLaunch*>(p);
-}
-void stem_free(StemLaunch* p) { free(p); }
+StemLaunch* stem_alloc() { return new (std::nothrow) StemLaunch(); }
+void stem_free(StemLaunch* p) { delete p; }
 
 int stem_prepare(const void* img, int img_dtype, const void* w, const float* bias, void* out, long long out_ld,
                  int batch, int h, int wd, int out_c, int act, int dtype, StemLaunch* L) {
@@ -360,8 +350,6 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
   YX_REQUIRE(out_c % 16 == 0 && out_c >= 16 && out_c <= 128, YX_ERR_UNSUPPORTED, "stem: out_c=%d (16..128, multiple of 16)", out_c);
   YX_REQUIRE(out_ld % 16 == 0 && out_ld >= out_c && ((uintptr_t)out & 31) == 0, YX_ERR_INVALID_ARG, "stem: out misaligned");
   YX_REQUIRE(((uintptr_t)img & 15) == 0 && ((uintptr_t)w & 15) == 0 && ((uintptr_t)bias & 15) == 0, YX_ERR_INVALID_ARG, "stem: pointer alignment");
-  EncodeTiledFn encode = get_encode_fn();
-  YX_REQUIRE(encode != nullptr, YX_ERR_NO_DEVICE, "cuTensorMapEncodeTiled unavailable (no CUDA driver)");
   StemParams& p = L->p;
   memset(&p, 0, sizeof(p));
   p.img = img; p.img_dtype = img_dtype; p.batch = batch; p.h = h; p.w = wd;
@@ -404,9 +392,8 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
   const int n_stages = V == 0 ? StemCfg<0>::kStages : StemCfg<1>::kStages;
   const int n_patch = V == 0 ? StemCfg<0>::kPatchStages : StemCfg<1>::kPatchStages;
   p.tmem_cols = (unsigned)(n_acc * p.BNpad);
-  const unsigned fmt = dtype == YX_BF16 ? 1u : 0u;
-  p.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((unsigned)(p.BN >> 3) << 17) | ((128u >> 4) << 24);
-  p.desc_hi = ((256u >> 4) & 0x3FFFu) | (1u << 14) | (6u << 29);    // SBO = 8 rows * 32 B, version 1, SWIZZLE_32B
+  p.idesc = umma_idesc(dtype, p.BN);
+  p.desc_hi = umma_desc_hi(32);                                      // 16 channels per tap: 32-byte rows
   p.bias_bytes = ((unsigned)out_c * 4u + 1023u) & ~1023u;
   p.w_tile_bytes = (unsigned)out_c * 32u;                            // one tap: [out_c x 16], a multiple of 512 B
   p.b_bytes = 9u * p.w_tile_bytes;
@@ -433,63 +420,41 @@ int stem_prepare(const void* img, int img_dtype, const void* w, const float* bia
     cuuint64_t idims[4] = {(cuuint64_t)wd, (cuuint64_t)h, 3, (cuuint64_t)batch};
     cuuint64_t istr[3] = {(cuuint64_t)wd * es, (cuuint64_t)wd * h * es, (cuuint64_t)wd * h * 3 * es};
     cuuint32_t ibox[4] = {bw, (cuuint32_t)p.patch_rows, 3, 1};
-    cuuint32_t iestr[4] = {1, 1, 1, 1};
-    CUresult ri = encode(&L->map_img, img_dtype == YX_FP32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 4,
-                         const_cast<void*>(img), idims, istr, ibox, iestr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    YX_REQUIRE(ri == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(stem image) failed: %d", (int)ri);
+    const int rc = encode_tma(&L->map_img, tma_dtype(img_dtype), 4, img, idims, istr, ibox, nullptr, CU_TENSOR_MAP_SWIZZLE_NONE,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "stem image");
+    if (rc) return rc;
     p.patch_tx = bw * (cuuint32_t)p.patch_rows * 3 * es;
   }
-  const CUtensorMapDataType tdt = dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   cuuint64_t dims[2] = {144, (cuuint64_t)out_c};
   cuuint64_t strides[1] = {288};
   cuuint32_t box[2] = {16, (cuuint32_t)out_c};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = encode(&L->map_w, tdt, 2, const_cast<void*>(w), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                      CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  YX_REQUIRE(r == CUDA_SUCCESS, YX_ERR_CUDA, "cuTensorMapEncodeTiled(stem W) failed: %d", (int)r);
+  const int rc = encode_tma(&L->map_w, tma_dtype(dtype), 2, w, dims, strides, box, nullptr, tma_swizzle(32),
+                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "stem W");
+  if (rc) return rc;
   const int sms = num_sms() * (V == 0 ? 1 : 2);
   L->grid = p.num_tiles < sms ? p.num_tiles : sms;
   return YX_OK;
 }
 
+// [variant][uint8 image][fp16 output][SiLU]
+static decltype(&stem_tc_kernel<float, false, false, 0>) const kStemKernels[2][2][2][2] = {
+    {{{stem_tc_kernel<float, false, false, 0>, stem_tc_kernel<float, false, true, 0>},
+      {stem_tc_kernel<float, true, false, 0>, stem_tc_kernel<float, true, true, 0>}},
+     {{stem_tc_kernel<uint8_t, false, false, 0>, stem_tc_kernel<uint8_t, false, true, 0>},
+      {stem_tc_kernel<uint8_t, true, false, 0>, stem_tc_kernel<uint8_t, true, true, 0>}}},
+    {{{stem_tc_kernel<float, false, false, 1>, stem_tc_kernel<float, false, true, 1>},
+      {stem_tc_kernel<float, true, false, 1>, stem_tc_kernel<float, true, true, 1>}},
+     {{stem_tc_kernel<uint8_t, false, false, 1>, stem_tc_kernel<uint8_t, false, true, 1>},
+      {stem_tc_kernel<uint8_t, true, false, 1>, stem_tc_kernel<uint8_t, true, true, 1>}}}};
+
 int stem_launch(const StemLaunch* L, cudaStream_t stream) {
-  static bool attr_set_dev[kMaxDevices] = {};
-  bool& attr_set = attr_set_dev[current_device_slot()];
-  if (!attr_set) {
-#define YX_STEM_ATTR1(T, F, V) \
-  YX_CUDA(cudaFuncSetAttribute(stem_tc_kernel<T, F, true, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, V == 0 ? 200 * 1024 : 112 * 1024)); \
-  YX_CUDA(cudaFuncSetAttribute(stem_tc_kernel<T, F, false, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, V == 0 ? 200 * 1024 : 112 * 1024))
-#define YX_STEM_ATTR(T, F) YX_STEM_ATTR1(T, F, 0); YX_STEM_ATTR1(T, F, 1)
-    YX_STEM_ATTR(float, false); YX_STEM_ATTR(float, true); YX_STEM_ATTR(uint8_t, false); YX_STEM_ATTR(uint8_t, true);
-#undef YX_STEM_ATTR
-#undef YX_STEM_ATTR1
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)L->grid);
+  static bool smem_set[kMaxDevices] = {};
+  // the first 8 kernels are variant 0 (one CTA per SM), the other 8 variant 1 (two CTAs per SM)
+  YX_CUDA(opt_in_smem(smem_set, kStemKernels, [](int i) { return i < 8 ? 200 * 1024 : 112 * 1024; }));
   const int V = L->variant;
-  cfg.blockDim = dim3((unsigned)(V == 0 ? StemCfg<0>::kThreads : StemCfg<1>::kThreads));
-  cfg.dynamicSmemBytes = L->smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const bool h16 = L->p.epi.dtype == YX_FP16;
-  const bool silu = L->p.epi.act == YX_ACT_SILU;
-#define YX_STEM_GO1(T, F, V) do { if (silu) YX_CUDA(cudaLaunchKernelEx(&cfg, stem_tc_kernel<T, F, true, V>, L->map_w, L->map_img, L->p)); \
-    else YX_CUDA(cudaLaunchKernelEx(&cfg, stem_tc_kernel<T, F, false, V>, L->map_w, L->map_img, L->p)); } while (0)
-#define YX_STEM_GO(T, F) do { if (V == 0) YX_STEM_GO1(T, F, 0); else YX_STEM_GO1(T, F, 1); } while (0)
-  if (L->p.img_dtype == YX_FP32) {
-    if (h16) YX_STEM_GO(float, true); else YX_STEM_GO(float, false);
-  } else {
-    if (h16) YX_STEM_GO(uint8_t, true); else YX_STEM_GO(uint8_t, false);
-  }
-#undef YX_STEM_GO
-#undef YX_STEM_GO1
+  const auto kernel = kStemKernels[V][L->p.img_dtype != YX_FP32][L->p.epi.dtype == YX_FP16][L->p.epi.act == YX_ACT_SILU];
+  YX_CUDA(launch_pdl(kernel, dim3((unsigned)L->grid), dim3((unsigned)(V == 0 ? StemCfg<0>::kThreads : StemCfg<1>::kThreads)),
+                     L->smem, stream, L->map_w, L->map_img, L->p));
   return YX_OK;
 }
 

@@ -21,18 +21,11 @@
 // sums the partials in a fixed order (deterministic, unlike atomics) into the gradient tensor with the weight's strides.
 //
 // One CTA = 6 warps: warp 0 TMA producer, warp 1 TMEM allocator + MMA issuer, warps 2..5 epilogue (tcgen05.ld -> global).
-#include <stdlib.h>
 #include <string.h>
 
 #include "yx_common.cuh"
 
 namespace yx {
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode_fn();   // yx_conv_tc.cu
 
 static constexpr int kWgStages = 4;
 
@@ -51,13 +44,6 @@ struct WgradParams {
   unsigned desc_hi_a, desc_hi_b, lbo_a16, lbo_b16, idesc;
   float* partial;
   long long split_stride, row_stride;   // elements
-};
-
-struct WgradLaunch {
-  CUtensorMap map_dy, map_x;
-  WgradParams p;
-  int grid;
-  size_t smem;
 };
 
 struct __align__(8) WgShared {
@@ -344,10 +330,7 @@ static int wgrad_plan(int batch, int in_h, int in_w, int in_c, int out_h, int ou
   p.n_groups = (p.slices + p.SG - 1) / p.SG;
   p.merged = (p.n_blocks == 1 && p.SG > 1 && p.SG * p.N <= 256) ? 1 : 0;
 
-  int dev = 0, max_smem = 0;
-  YX_CUDA(cudaGetDevice(&dev));
-  YX_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  const int budget = max_smem - 4096;                    // 1 KB alignment slack + static shared (barriers)
+  const int budget = max_smem_optin() - 4096;                   // 1 KB alignment slack + static shared (barriers)
   const unsigned bpp = 256u + (unsigned)(p.SG * p.N) * 2u;   // bytes per pixel of one stage: 128 A channels + SG * N B channels
   int kp_max = (budget / 3) / (int)bpp / 16 * 16;
   if (kp_max > 128) kp_max = 128;
@@ -395,11 +378,6 @@ long long wgrad_ws_bytes(int batch, int in_h, int in_w, int in_c, int out_h, int
   return (long long)p.ksplit * p.split_stride * 4;
 }
 
-static unsigned layout_code(unsigned rb) { return rb == 128 ? 2u : (rb == 64 ? 4u : 6u); }   // SW128 / SW64 / SW32
-static CUtensorMapSwizzle swizzle_of(unsigned rb) {
-  return rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (rb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-}
-
 int wgrad_launch(const void* x, long long x_ld, const void* dy, long long dy_ld, int dtype, int batch, int in_h, int in_w, int in_c,
                  int out_h, int out_w, int out_c, int ksize, int stride, int in_c_real, int out_c_real, float* dw, long long dw_so,
                  long long dw_si, long long dw_st, int accumulate, void* ws, long long ws_bytes, cudaStream_t stream) {
@@ -408,67 +386,49 @@ int wgrad_launch(const void* x, long long x_ld, const void* dy, long long dy_ld,
   YX_REQUIRE(x_ld % 8 == 0 && dy_ld % 8 == 0 && ((uintptr_t)x & 15) == 0 && ((uintptr_t)dy & 15) == 0, YX_ERR_INVALID_ARG,
              "wgrad: activations must be 16-byte aligned with a pixel stride that is a multiple of 8");
   YX_REQUIRE(in_c_real > 0 && in_c_real <= in_c && out_c_real > 0 && out_c_real <= out_c, YX_ERR_INVALID_ARG, "wgrad: real channel counts");
-  WgradLaunch* L = nullptr;
-  if (posix_memalign(reinterpret_cast<void**>(&L), 64, sizeof(WgradLaunch)) != 0) { set_error("wgrad: out of host memory"); return YX_ERR_INVALID_ARG; }
-  int rc = wgrad_plan(batch, in_h, in_w, in_c, out_h, out_w, out_c, ksize, stride, &L->p, &L->smem);
-  if (rc) { free(L); return rc; }
-  WgradParams& p = L->p;
-  if ((long long)p.ksplit * p.split_stride * 4 > ws_bytes) {
-    set_error("wgrad: workspace of %lld bytes, need %lld", ws_bytes, (long long)p.ksplit * p.split_stride * 4);
-    free(L); return YX_ERR_CAPACITY;
-  }
+  WgradParams p;
+  size_t smem = 0;
+  int rc = wgrad_plan(batch, in_h, in_w, in_c, out_h, out_w, out_c, ksize, stride, &p, &smem);
+  if (rc) return rc;
+  YX_REQUIRE((long long)p.ksplit * p.split_stride * 4 <= ws_bytes, YX_ERR_CAPACITY, "wgrad: workspace of %lld bytes, need %lld",
+             ws_bytes, (long long)p.ksplit * p.split_stride * 4);
   p.partial = reinterpret_cast<float*>(ws);
   p.lbo_a16 = p.a_block_bytes >> 4;
   p.lbo_b16 = p.b_block_bytes >> 4;
-  p.desc_hi_a = (((8u * p.rb_a) >> 4) & 0x3FFFu) | (1u << 14) | (layout_code(p.rb_a) << 29);
-  p.desc_hi_b = (((8u * p.rb_b) >> 4) & 0x3FFFu) | (1u << 14) | (layout_code(p.rb_b) << 29);
-  const unsigned fmt = dtype == YX_BF16 ? 1u : 0u;
-  // fp32 accumulate | A, B formats | A and B MN-major (bits 15, 16) | N >> 3 | M >> 4
-  p.idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (1u << 15) | (1u << 16) | ((unsigned)(p.N >> 3) << 17) | ((128u >> 4) << 24);
+  p.desc_hi_a = umma_desc_hi(p.rb_a);
+  p.desc_hi_b = umma_desc_hi(p.rb_b);
+  p.idesc = umma_idesc(dtype, p.N, /*mn_major=*/true);
 
-  EncodeTiledFn encode = get_encode_fn();
-  if (!encode) { set_error("cuTensorMapEncodeTiled unavailable (no CUDA driver)"); free(L); return YX_ERR_NO_DEVICE; }
-  const CUtensorMapDataType tdt = dtype == YX_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  CUtensorMap map_dy, map_x;
   {
     cuuint64_t dims[4] = {(cuuint64_t)out_c, (cuuint64_t)out_w, (cuuint64_t)out_h, (cuuint64_t)batch};
     cuuint64_t strides[3] = {(cuuint64_t)dy_ld * 2, (cuuint64_t)dy_ld * 2 * out_w, (cuuint64_t)dy_ld * 2 * out_w * out_h};
     cuuint32_t box[4] = {(cuuint32_t)p.co_box, (cuuint32_t)p.tw, (cuuint32_t)p.th, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&L->map_dy, tdt, 4, const_cast<void*>(dy), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        swizzle_of(p.rb_a), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("wgrad: cuTensorMapEncodeTiled(dy) failed: %d", (int)r); free(L); return YX_ERR_CUDA; }
+    rc = encode_tma(&map_dy, tma_dtype(dtype), 4, dy, dims, strides, box, nullptr, tma_swizzle(p.rb_a),
+                    CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "wgrad dy");
+    if (rc) return rc;
   }
   {
     cuuint64_t dims[4] = {(cuuint64_t)in_c, (cuuint64_t)in_w, (cuuint64_t)in_h, (cuuint64_t)batch};
     cuuint64_t strides[3] = {(cuuint64_t)x_ld * 2, (cuuint64_t)x_ld * 2 * in_w, (cuuint64_t)x_ld * 2 * in_w * in_h};
     cuuint32_t box[4] = {(cuuint32_t)p.ci_box, (cuuint32_t)(p.tw * stride), (cuuint32_t)(p.th * stride), 1};
     cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
-    CUresult r = encode(&L->map_x, tdt, 4, const_cast<void*>(x), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        swizzle_of(p.rb_b), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("wgrad: cuTensorMapEncodeTiled(x) failed: %d", (int)r); free(L); return YX_ERR_CUDA; }
+    rc = encode_tma(&map_x, tma_dtype(dtype), 4, x, dims, strides, box, estr, tma_swizzle(p.rb_b), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                    "wgrad x");
+    if (rc) return rc;
   }
-  static bool attr_set_dev[kMaxDevices] = {};
-  bool& attr_set = attr_set_dev[current_device_slot()];
-  if (!attr_set) {
-    int dev = 0, max_smem = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    cudaFuncAttributes fa;
+  static bool smem_set[kMaxDevices] = {};
+  YX_CUDA(opt_in_smem(smem_set, &wgrad_tc_kernel, [](int) {
+    cudaFuncAttributes fa = {};
     cudaFuncGetAttributes(&fa, wgrad_tc_kernel);             // the opt-in limit covers static + dynamic shared memory
-    cudaError_t e = cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - (int)fa.sharedSizeBytes);
-    if (e != cudaSuccess) { free(L); return cuda_fail(e, "cudaFuncSetAttribute(wgrad_tc_kernel)", __FILE__, __LINE__); }
-    attr_set = true;
-  }
+    return max_smem_optin() - (int)fa.sharedSizeBytes;
+  }));
   const int grid = p.m_tiles * p.n_groups * p.ksplit;
-  cudaError_t e = launch_kernel(wgrad_tc_kernel, dim3(grid), dim3(192), L->smem, stream, L->map_dy, L->map_x, p);
-  if (e == cudaSuccess) {
-    const long long total = (long long)out_c * p.taps * in_c;
-    const int rgrid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-    e = launch_kernel(wgrad_reduce_kernel, dim3(rgrid), dim3(256), 0, stream, (const float*)p.partial, p.ksplit, p.split_stride, p.row_stride,
-                   p.N, p.taps, out_c, in_c, out_c_real, in_c_real, dw, dw_so, dw_si, dw_st, accumulate);
-  }
-  free(L);
-  if (e != cudaSuccess) return cuda_fail(e, "wgrad launch", __FILE__, __LINE__);
+  YX_CUDA(launch_kernel(wgrad_tc_kernel, dim3(grid), dim3(192), smem, stream, map_dy, map_x, p));
+  const long long total = (long long)out_c * p.taps * in_c;
+  const int rgrid = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
+  YX_CUDA(launch_kernel(wgrad_reduce_kernel, dim3(rgrid), dim3(256), 0, stream, (const float*)p.partial, p.ksplit, p.split_stride,
+                        p.row_stride, p.N, p.taps, out_c, in_c, out_c_real, in_c_real, dw, dw_so, dw_si, dw_st, accumulate));
   return YX_OK;
 }
 
