@@ -422,6 +422,32 @@ int yx_pack_train_weights_multi(const int64_t* table, const int32_t* chunks, int
                                 void* stream);
 int yx_dilate2(const void* dy, void* z, int32_t batch, int32_t oh, int32_t ow, int32_t zh, int32_t zw, int32_t c, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Training depthwise conv (the depthwise BaseConv of DWConv, yolox/models/network_blocks.py:55-74, inside the training step):
+ * 3x3, pad 1, no bias, stride 1 | 2, groups = channels = c. Output size oh = (in_h - 1) / stride + 1, ow likewise.
+ *   forward : yx_dwconv3x3_train_fwd, y[b, p, c] = sum over taps of x[b, p*stride + tap - 1, c] * w16[c, tap]
+ *   dgrad   : yx_dwconv3x3_dgrad, dx[b, q, c] = sum over the taps where (q + 1 - tap) / stride is exact and inside dy of
+ *             dy[b, (q + 1 - tap) / stride, c] * w16[c, tap] (a gather: no atomics, no zero-stuffed copy)
+ *   wgrad   : yx_dwconv3x3_wgrad, dW[c, tap] = sum over b and output pixels p of dy[b, p, c] * x[b, p*stride + tap - 1, c]: the
+ *             pixels split over CTAs (the split depends on the shape and the device only), fp32 partials [split][9][c] in the
+ *             caller's workspace (yx_dwconv3x3_wgrad_workspace_bytes; -1 for a bad shape), summed in split order by a second
+ *             launch: deterministic. accumulate != 0: dw += (straight into the parameter's .grad).
+ * w / dw: the fp32 parameter [c, 1, 3, 3], element (c, tap = 3*kh + kw) at c*w_stride_c + tap*w_stride_tap, so NCHW-contiguous and
+ * channels_last weights both work. The forward and the dgrad round w to `dtype` as they read it (autocast's weight cast).
+ * x, y, dy, dx: NHWC, dtype YX_BF16 | YX_FP16, per-pixel strides *_ld in elements (multiples of 8, >= c), 16-byte aligned;
+ * c % 8 == 0. fp32 accumulation. A bad shape or pointer returns a negative yx_status (message: yx_last_error()).
+ * ------------------------------------------------------------------------------------------ */
+int yx_dwconv3x3_train_fwd(const void* x, int64_t x_ld, const float* w, int64_t w_stride_c, int64_t w_stride_tap, void* y,
+                           int64_t y_ld, int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride, int32_t dtype,
+                           void* stream);
+int yx_dwconv3x3_dgrad(const void* dy, int64_t dy_ld, const float* w, int64_t w_stride_c, int64_t w_stride_tap, void* dx,
+                       int64_t dx_ld, int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride, int32_t dtype,
+                       void* stream);
+int64_t yx_dwconv3x3_wgrad_workspace_bytes(int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride);
+int yx_dwconv3x3_wgrad(const void* x, int64_t x_ld, const void* dy, int64_t dy_ld, int32_t dtype, int32_t batch, int32_t in_h,
+                       int32_t in_w, int32_t c, int32_t stride, float* dw, int64_t dw_stride_c, int64_t dw_stride_tap,
+                       int32_t accumulate, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* Backward of the SPP pools (SPPBottleneck, network_blocks.py:120-142; forward = yx_spp_maxpool on the concat buffer):
  * cat: NHWC buffer whose channels [0, c) hold the pools' input x (pixel stride ld); dout: NHWC gradient of the 4c-channel
  * concat (pixel stride dout_ld); dx32: dense fp32 [B, h, w, c] that the CALLER pre-loads with dout[..., :c] (the identity

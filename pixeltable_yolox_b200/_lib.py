@@ -105,6 +105,10 @@ SIGNATURES = {
     "yx_spp_maxpool_bwd": (C.c_int, [_P, _I64, _P, _I64, _P, _I32, _I32, _I32, _I32, _I32, _P]),
     "yx_pack_train_weights_multi": (C.c_int, [_P, _P, _I32, _I32, _I32, _P]),
     "yx_dilate2": (C.c_int, [_P, _P, _I32, _I32, _I32, _I32, _I32, _I32, _P]),
+    "yx_dwconv3x3_train_fwd": (C.c_int, [_P, _I64, _P, _I64, _I64, _P, _I64] + [_I32] * 6 + [_P]),
+    "yx_dwconv3x3_dgrad": (C.c_int, [_P, _I64, _P, _I64, _I64, _P, _I64] + [_I32] * 6 + [_P]),
+    "yx_dwconv3x3_wgrad_workspace_bytes": (_I64, [_I32] * 5),
+    "yx_dwconv3x3_wgrad": (C.c_int, [_P, _I64, _P, _I64] + [_I32] * 6 + [_P, _I64, _I64, _I32, _P, _I64, _P]),
     "yx_letterbox_u8": (C.c_int, [_P, _I32, _I32, _I32, _I32, _P, _I32, _P]),
     "yx_coco_rows": (C.c_int, [_P, _P, _I32, _I32, _P, _P, _P, _I32, _P, _P, _P, _P, _P, _P]),
     "yx_plan_create": (_P, []),

@@ -20,7 +20,8 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libyx_b200.so"
 OBJ_DIR = PKG / "build"
-SOURCES = ["yx_api.cu", "yx_conv_tc.cu", "yx_bneck_tc.cu", "yx_stem_tc.cu", "yx_conv_simt.cu", "yx_misc.cu", "yx_postprocess.cu", "yx_simota.cu", "yx_losses.cu", "yx_train.cu", "yx_preproc.cu", "yx_wgrad_tc.cu", "yx_allreduce_sgd.cu"]
+SOURCES = ["yx_api.cu", "yx_conv_tc.cu", "yx_bneck_tc.cu", "yx_stem_tc.cu", "yx_conv_simt.cu", "yx_misc.cu", "yx_postprocess.cu", "yx_simota.cu", "yx_losses.cu", "yx_train.cu", "yx_preproc.cu", "yx_wgrad_tc.cu", "yx_allreduce_sgd.cu",
+           "yx_dwconv_train.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

@@ -76,6 +76,14 @@ int wgrad_launch(const void* x, long long x_ld, const void* dy, long long dy_ld,
 int pack_train_weights_launch(const float* w, long long so, long long si, long long st, int o, int i, int taps, int o_pad, int i_pad,
                               void* wf, void* wd, int subpixel, int dtype, cudaStream_t stream);
 int dilate2_launch(const void* dy, void* z, int batch, int oh, int ow, int zh, int zw, int c, cudaStream_t stream);
+int dw_train_fwd_launch(const void* x, long long x_ld, const float* w, long long w_sc, long long w_st, void* y, long long y_ld,
+                        int batch, int in_h, int in_w, int c, int stride, int dtype, cudaStream_t stream);
+int dw_dgrad_launch(const void* dy, long long dy_ld, const float* w, long long w_sc, long long w_st, void* dx, long long dx_ld,
+                    int batch, int in_h, int in_w, int c, int stride, int dtype, cudaStream_t stream);
+long long dw_wgrad_ws_bytes(int batch, int in_h, int in_w, int c, int stride);
+int dw_wgrad_launch(const void* x, long long x_ld, const void* dy, long long dy_ld, int dtype, int batch, int in_h, int in_w, int c,
+                    int stride, float* dw, long long dw_sc, long long dw_st, int accumulate, void* ws, long long ws_bytes,
+                    cudaStream_t stream);
 int pack_train_weights_multi_launch(const long long* table, const int* chunks, int n_chunks, int chunk_elems, int dtype, cudaStream_t stream);
 int spp_bwd_launch(const void* cat, long long ld, const void* dout, long long dld, float* dx32, int batch, int h, int w, int c,
                    int dtype, cudaStream_t s);
@@ -547,6 +555,36 @@ int yx_dilate2(const void* dy, void* z, int32_t batch, int32_t oh, int32_t ow, i
   int rc = require_device();
   if (rc) return rc;
   return dilate2_launch(dy, z, batch, oh, ow, zh, zw, c, (cudaStream_t)stream);
+}
+
+int yx_dwconv3x3_train_fwd(const void* x, int64_t x_ld, const float* w, int64_t w_stride_c, int64_t w_stride_tap, void* y,
+                           int64_t y_ld, int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride, int32_t dtype,
+                           void* stream) {
+  int rc = require_device();
+  if (rc) return rc;
+  return dw_train_fwd_launch(x, x_ld, w, w_stride_c, w_stride_tap, y, y_ld, batch, in_h, in_w, c, stride, dtype, (cudaStream_t)stream);
+}
+
+int yx_dwconv3x3_dgrad(const void* dy, int64_t dy_ld, const float* w, int64_t w_stride_c, int64_t w_stride_tap, void* dx,
+                       int64_t dx_ld, int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride, int32_t dtype,
+                       void* stream) {
+  int rc = require_device();
+  if (rc) return rc;
+  return dw_dgrad_launch(dy, dy_ld, w, w_stride_c, w_stride_tap, dx, dx_ld, batch, in_h, in_w, c, stride, dtype, (cudaStream_t)stream);
+}
+
+int64_t yx_dwconv3x3_wgrad_workspace_bytes(int32_t batch, int32_t in_h, int32_t in_w, int32_t c, int32_t stride) {
+  if (require_device()) return -1;
+  return dw_wgrad_ws_bytes(batch, in_h, in_w, c, stride);
+}
+
+int yx_dwconv3x3_wgrad(const void* x, int64_t x_ld, const void* dy, int64_t dy_ld, int32_t dtype, int32_t batch, int32_t in_h,
+                       int32_t in_w, int32_t c, int32_t stride, float* dw, int64_t dw_stride_c, int64_t dw_stride_tap,
+                       int32_t accumulate, void* workspace, int64_t workspace_bytes, void* stream) {
+  int rc = require_device();
+  if (rc) return rc;
+  return dw_wgrad_launch(x, x_ld, dy, dy_ld, dtype, batch, in_h, in_w, c, stride, dw, dw_stride_c, dw_stride_tap, accumulate,
+                         workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int yx_letterbox_u8(const yx_letterbox_image* images, int32_t batch, int32_t channels, int32_t H, int32_t W, void* out,

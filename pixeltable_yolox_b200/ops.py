@@ -702,6 +702,77 @@ def conv_wgrad(x: torch.Tensor, dy: torch.Tensor, weight_like: torch.Tensor, ksi
     return dw
 
 
+def _dw_weight_strides(w: torch.Tensor):
+    """(stride_c, stride_tap) of a depthwise conv weight (or its gradient) [c, 1, 3, 3]."""
+    assert w.dim() == 4 and w.shape[1:] == (1, 3, 3) and w.dtype == torch.float32, (w.shape, w.dtype)
+    sc, _, st = _weight_strides(w)
+    return sc, st
+
+
+def dwconv_train_fwd(x: torch.Tensor, weight: torch.Tensor, stride: int) -> torch.Tensor:
+    """Depthwise 3x3 conv (pad 1, no bias) of the training step: x [B, c, H, W] 16-bit dense channels_last, weight the fp32
+    parameter [c, 1, 3, 3] (any strides; rounded to x's dtype as the kernel reads it) -> y [B, c, OH, OW] channels_last."""
+    require_cuda(x, "dwconv_train_fwd")
+    dev = x.device
+    same_device(dev, "dwconv_train_fwd", weight=weight)
+    xv = _nhwc(x)
+    sc, st = _dw_weight_strides(weight)
+    assert weight.shape[0] == xv.c and x.dtype in (torch.bfloat16, torch.float16)
+    oh, ow = (xv.H - 1) // stride + 1, (xv.W - 1) // stride + 1
+    y = torch.empty((xv.B, xv.c, oh, ow), dtype=x.dtype, device=dev, memory_format=torch.channels_last)
+    yv = _nhwc(y)
+    with on_device(dev):
+        check(lib().yx_dwconv3x3_train_fwd(xv.ptr, xv.ld, weight.data_ptr(), sc, st, yv.ptr, yv.ld, xv.B, xv.H, xv.W, xv.c, stride,
+                                           dtype_code(x.dtype), stream_ptr(dev)), "dwconv3x3_train_fwd")
+    return y
+
+
+def dwconv_dgrad(dy: torch.Tensor, weight: torch.Tensor, stride: int, in_h: int, in_w: int) -> torch.Tensor:
+    """Input gradient of dwconv_train_fwd: dy [B, c, OH, OW] 16-bit dense channels_last -> dx [B, c, in_h, in_w] (same)."""
+    require_cuda(dy, "dwconv_dgrad")
+    dev = dy.device
+    same_device(dev, "dwconv_dgrad", weight=weight)
+    dv = _nhwc(dy)
+    sc, st = _dw_weight_strides(weight)
+    assert weight.shape[0] == dv.c and dy.dtype in (torch.bfloat16, torch.float16)
+    assert (dv.H, dv.W) == ((in_h - 1) // stride + 1, (in_w - 1) // stride + 1), ((dv.H, dv.W), (in_h, in_w), stride)
+    dx = torch.empty((dv.B, dv.c, in_h, in_w), dtype=dy.dtype, device=dev, memory_format=torch.channels_last)
+    xv = _nhwc(dx)
+    with on_device(dev):
+        check(lib().yx_dwconv3x3_dgrad(dv.ptr, dv.ld, weight.data_ptr(), sc, st, xv.ptr, xv.ld, xv.B, in_h, in_w, xv.c, stride,
+                                       dtype_code(dy.dtype), stream_ptr(dev)), "dwconv3x3_dgrad")
+    return dx
+
+
+def dwconv_wgrad(x: torch.Tensor, dy: torch.Tensor, weight_like: torch.Tensor, stride: int,
+                 accumulate_into: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Weight gradient of dwconv_train_fwd: x [B, c, H, W] and dy [B, c, OH, OW], both 16-bit dense channels_last -> fp32 dW
+    with weight_like's shape [c, 1, 3, 3] and strides; deterministic. accumulate_into: an fp32 tensor of the weight's shape
+    (its .grad): dW is ADDED to it in place and returned."""
+    require_cuda(x, "dwconv_wgrad")
+    dev = x.device
+    same_device(dev, "dwconv_wgrad", dy=dy, weight=weight_like)
+    xv, dv = _nhwc(x), _nhwc(dy)
+    assert x.dtype == dy.dtype and x.dtype in (torch.bfloat16, torch.float16)
+    assert xv.B == dv.B and xv.c == dv.c == weight_like.shape[0]
+    assert (dv.H, dv.W) == ((xv.H - 1) // stride + 1, (xv.W - 1) // stride + 1)
+    if accumulate_into is not None:
+        dw = accumulate_into
+        assert dw.dtype == torch.float32 and dw.shape == weight_like.shape and dw.device == dev
+    else:
+        dw = torch.empty_strided(weight_like.shape, weight_like.stride(), dtype=torch.float32, device=dev)
+    sc, st = _dw_weight_strides(dw)
+    nbytes = lib().yx_dwconv3x3_wgrad_workspace_bytes(xv.B, xv.H, xv.W, xv.c, stride)
+    if nbytes < 0:
+        check(-1, "dwconv3x3_wgrad (workspace query)")
+    ws = _workspace(dev, nbytes, f"wgrad:{stream_ptr(dev)}")        # per stream, shared with conv_wgrad (same-stream launches serialise)
+    with on_device(dev):
+        check(lib().yx_dwconv3x3_wgrad(xv.ptr, xv.ld, dv.ptr, dv.ld, dtype_code(x.dtype), xv.B, xv.H, xv.W, xv.c, stride,
+                                       dw.data_ptr(), sc, st, 0 if accumulate_into is None else 1, ws.data_ptr(), ws.numel(),
+                                       stream_ptr(dev)), "dwconv3x3_wgrad")
+    return dw
+
+
 def dilate2(dy: torch.Tensor, zh: int, zw: int) -> torch.Tensor:
     """Zero-stuffed copy of dy [B, C, OH, OW] (channels_last): z [B, C, zh, zw] with z[..., 2*oy, 2*ox] = dy[..., oy, ox]."""
     require_cuda(dy, "dilate2")

@@ -11,6 +11,10 @@ prediction convs (yolox/models/yolo_head.py:94-120) inside `Trainer.train_one_it
 Activations stay 16-bit channels_last (NHWC) between layers, which is the layout every kernel of this package uses; the
 fp32 master weights are packed to 16-bit operands once per step (WeightPacker: one launch for all layers; without it one
 launch per layer for the forward and the dgrad operand). Numerics match torch.autocast: 16-bit operands, fp32 accumulation, fp32 weight gradients.
+
+Depthwise 3x3 convs (groups == channels, the first half of DWConv in yolox_nano) run on SIMT kernels instead
+(csrc/yx_dwconv_train.cu: forward and dgrad as one gather kernel, wgrad as a deterministic split reduction); they read the fp32
+master weight directly, so they need no packed operands.
 """
 from __future__ import annotations
 
@@ -194,6 +198,53 @@ def usable(x: torch.Tensor, conv: torch.nn.Conv2d) -> Optional[torch.dtype]:
     return dt if dt in (torch.bfloat16, torch.float16) else None
 
 
+def usable_depthwise(x: torch.Tensor, conv: torch.nn.Conv2d) -> Optional[torch.dtype]:
+    """The 16-bit compute dtype when this conv can run on the depthwise training kernels, else None (torch / cuDNN runs it):
+    CUDA, groups == in == out channels (a multiple of 8), 3x3 stride 1 / 2, pad 1, no bias, fp32 weight, under 16-bit
+    autocast or on 16-bit input."""
+    if os.environ.get("YX_TRAIN_CONV", "1") == "0" or not x.is_cuda or x.dim() != 4:
+        return None
+    c = conv.in_channels
+    if conv.groups != c or conv.out_channels != c or c % 8 != 0 or x.shape[1] != c or conv.bias is not None:
+        return None
+    if conv.kernel_size != (3, 3) or conv.stride not in ((1, 1), (2, 2)) or conv.padding != (1, 1):
+        return None
+    if conv.dilation != (1, 1) or conv.padding_mode != "zeros" or conv.weight.dtype != torch.float32:
+        return None
+    dt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
+    return dt if dt in (torch.bfloat16, torch.float16) else None
+
+
+class _DwConv(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, stride, dtype):
+        xh = x.detach().to(dtype).contiguous(memory_format=torch.channels_last)
+        y = ops.dwconv_train_fwd(xh, weight.detach(), stride)
+        ctx.save_for_backward(xh, weight)
+        ctx.geom = (stride, x.dtype)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xh, weight = ctx.saved_tensors
+        stride, x_dtype = ctx.geom
+        dyh = dy.to(xh.dtype).contiguous(memory_format=torch.channels_last)
+        dx = dw = None
+        if ctx.needs_input_grad[1]:
+            target = direct_target(weight)
+            if target is not None:
+                stream, pending = _side(xh.device)
+                stream.wait_event(torch.cuda.current_stream(xh.device).record_event())
+                with torch.cuda.stream(stream):
+                    ops.dwconv_wgrad(xh, dyh, weight, stride, accumulate_into=target)
+                pending.append((xh, dyh))
+            else:
+                dw = ops.dwconv_wgrad(xh, dyh, weight, stride)
+        if ctx.needs_input_grad[0]:
+            dx = ops.dwconv_dgrad(dyh, weight.detach(), stride, xh.shape[2], xh.shape[3]).to(x_dtype)
+        return dx, dw, None, None
+
+
 class _ConvTc(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias, stride, dtype):
@@ -277,8 +328,12 @@ class packed_weights:
 
 
 def conv2d(x: torch.Tensor, conv: torch.nn.Conv2d) -> torch.Tensor:
-    """`conv(x)` in the training step: tcgen05 forward / dgrad / wgrad when `usable`, else the module's own forward."""
+    """`conv(x)` in the training step: tcgen05 forward / dgrad / wgrad when `usable`, the depthwise kernels when
+    `usable_depthwise`, else the module's own forward."""
     dt = usable(x, conv)
-    if dt is None:
-        return conv(x)
-    return _ConvTc.apply(x, conv.weight, conv.bias, conv.stride[0], dt)
+    if dt is not None:
+        return _ConvTc.apply(x, conv.weight, conv.bias, conv.stride[0], dt)
+    dt = usable_depthwise(x, conv)
+    if dt is not None:
+        return _DwConv.apply(x, conv.weight, conv.stride[0], dt)
+    return conv(x)
